@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the chowdsp_fft hot path on B200 (DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  Default workload =
 BASELINE.json configs[1]: batched complex C2C N=4096 x 65536 transforms fp32, ordered, 1 GPU
@@ -138,6 +138,10 @@ class BatchedFFT:
 
     def step(self, stream):
         self.cf.fft_transform_batched(self.plan, self.x, self.y, self.batch, self.nfl, self.nfl, self.cf.FFT_FORWARD, self.ordered, stream)
+
+    def outputs(self):
+        """what one step hands its caller, each array as rows of its last dimension (--dump-outputs samples rows)"""
+        return {"y": self.y}
 
     def parity(self):
         from oracle import oracle as o
@@ -304,6 +308,9 @@ class ISTFT(STFT):
         self.cf.fft_istft_overlap_add(self.plan, self.spec, self.out, self.channels, self.frames, self.frames * self.N, self.N,
                                       self.samples, self.hop, self.win, 1.0 / self.N, True, stream)
 
+    def outputs(self):
+        return {"out": self.out}
+
     def parity(self):
         from oracle import oracle as o
 
@@ -370,6 +377,11 @@ class Reverb(BatchedFFT):
         self.cf.fft_partitioned_convolve_step(self.plan, win.data_ptr(), self.sig.shape[1], self.h, self.P * self.N, self.fdl, self.P * self.N,
                                               out.data_ptr(), self.out.shape[1], self.channels, self.P, t, 1.0 / self.N, stream)
         self.t += 1
+
+    def outputs(self):
+        """the block the last step produced for every channel"""
+        tb = (self.t - 1) % self.blocks
+        return {"out": self.out[:, tb * self.B:(tb + 1) * self.B]}
 
     def parity(self):
         """Last timed block of two channels against the oracle's composition of the same reference calls."""
@@ -530,6 +542,12 @@ class Huge(BatchedFFT):
             out = None if (self.natural and self.exchange == "peer") else self.y
             self.d.forward(self.x, out, stream=stream, natural=self.natural)
 
+    def outputs(self):
+        """complex bins as rows of (re, im)"""
+        # the natural-order peer exchange leaves its result in the distributed context, not in self.y
+        assert not (self.natural and self.exchange == "peer"), "no caller-visible output to dump for this variant"
+        return {"y": self.y.view(-1, 2)}
+
     def after_timing(self):
         """one extra, event-timed transform for the per-phase split (peer exchange only); it also fills self.y for the parity gate"""
         if self.world > 1 and self.exchange == "peer":
@@ -681,6 +699,9 @@ class Single1024(BatchedFFT):
         cf.fft_transform_batched(self.plan, self.x, self.y, 1, self.N, self.N, cf.FFT_FORWARD, True, stream)
         cf.fft_transform_batched(self.plan, self.y, self.z, 1, self.N, self.N, cf.FFT_BACKWARD, True, stream)
 
+    def outputs(self):
+        return {"y": self.y, "z": self.z}
+
     def parity(self):
         from oracle import oracle as o
 
@@ -760,9 +781,28 @@ def load_traffic(name, kernel_name):
     return ent.get("bytes"), ent.get("source")
 
 
-def measure(wl, name, ctx, steps, warmup, do_e2e, do_cpu, cpu_seconds, tune=None):
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(torch, outputs, out_dir):
+    """Writes every output as out_dir/<name>.npy (float32).  An output larger than its share of DUMP_BYTES is cut down to
+    a sample of its rows that depends only on its shape (the same rows on every run, in row order), so that two builds
+    run with the same arguments can be compared array for array."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(outputs)
+    for name, t in outputs.items():
+        if t.numel() * 4 > share:
+            rows = t.reshape(-1, t.shape[-1])
+            keep = share // (rows.shape[1] * 4)
+            idx = np.unique(np.random.default_rng(0).integers(0, rows.shape[0], keep))
+            t = rows[torch.from_numpy(idx).to(rows.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
+def measure(wl, name, ctx, steps, warmup, do_e2e, do_cpu, cpu_seconds, tune=None, dump_dir=None):
     """warm-up, `steps` timed steps (CUDA events on the launch stream, barrier + synchronize on both sides, max over
-    ranks), parity gate, e2e with host buffers, CPU baseline -> one record"""
+    ranks), outputs of the last step to `dump_dir` (rank 0), parity check, e2e with host buffers, CPU baseline -> one
+    record"""
     cf, torch, dist = ctx["cf"], ctx["torch"], ctx["dist"]
     rank, world, local_rank = ctx["rank"], ctx["world"], ctx["local_rank"]
     barrier, reduce_max, reduce_sum = ctx["barrier"], ctx["reduce_max"], ctx["reduce_sum"]
@@ -788,6 +828,8 @@ def measure(wl, name, ctx, steps, warmup, do_e2e, do_cpu, cpu_seconds, tune=None
     value = bytes_job / (ms_step * 1e-3) / 1e9
     per_gpu = wl.bytes_step / (ms_local * 1e-3) / 1e9
     peak, peak_src = hbm_peak()
+    if dump_dir is not None and rank == 0:
+        dump_outputs(torch, wl.outputs(), dump_dir)
     if hasattr(wl, "after_timing"):
         wl.after_timing()
 
@@ -840,15 +882,24 @@ def release(wl, torch):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline and of every sub-record (the e2e leg with host buffers times max(2, min(5, K)) calls)")
+    ap.add_argument("--warmup", type=int, default=3, help="warm-up steps before the timed ones, at least 3 whatever the value")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=None, choices=sorted(WORKLOADS), help="one workload only (default: the headline c2c4096 plus sub-records of every BASELINE config)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="headline workload only, no per-config sub-records")
     ap.add_argument("--tune", action="append", default=[], metavar="KEY=VALUE", help="fft_b200_set_tuning hook (sweeps only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline workload's outputs of its last timed step as DIR/<name>.npy (float32, at most 64 MB "
+                         "in all: a fixed sample of rows of larger outputs); inputs are seeded, so runs with the same arguments compare. "
+                         "With --gpus > 1, rank 0's share only, in the layout its step leaves it")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has no such outputs")
     headline = args.workload or "c2c4096"
     wl = WORKLOADS[headline]()
     rank = int(os.environ.get("RANK", "0"))
@@ -901,27 +952,28 @@ def main():
         k, v = kv.split("=")
         cf.set_tuning(k, int(v, 0))
     t_start = time.perf_counter()
-    line = measure(wl, headline, ctx, args.steps, args.warmup, not args.no_e2e, world == 1 and not args.no_cpu, 12.0, args.tune)
+    line = measure(wl, headline, ctx, args.steps, args.warmup, not args.no_e2e, world == 1 and not args.no_cpu, 12.0, args.tune,
+                   args.dump_outputs)
     release(wl, torch)
 
     # ---------------------------------------------------------------- sub-records: every BASELINE config in the driver-run line
     if args.workload is None and not args.no_configs:
         subs = []
         if world == 1:
-            plan = [("configs[0] single real N=1024 round trip (latency)", "single1024", Single1024, 20),
-                    ("configs[1] unordered half", "c2c4096_unordered", WORKLOADS["c2c4096_unordered"], 10),
-                    ("configs[2] STFT", "stft", STFT, 5),
-                    ("configs[3] reverb", "reverb", Reverb, 10),
-                    ("configs[4] N=2^28 on one GPU", "huge", Huge, 5)]
+            plan = [("configs[0] single real N=1024 round trip (latency)", "single1024", Single1024),
+                    ("configs[1] unordered half", "c2c4096_unordered", WORKLOADS["c2c4096_unordered"]),
+                    ("configs[2] STFT", "stft", STFT),
+                    ("configs[3] reverb", "reverb", Reverb),
+                    ("configs[4] N=2^28 on one GPU", "huge", Huge)]
         else:
-            plan = [("configs[2] STFT, channels sharded (strong scaling)", "stft", STFT, 5),
-                    ("configs[4] N=2^28 distributed, fused peer exchange, transposed-out", "huge", lambda: Huge(exchange="peer"), 10),
-                    ("configs[4] N=2^28 distributed, fused peer exchange, natural order (second all-to-all fused)", "huge", lambda: Huge(natural=True, exchange="peer"), 10),
-                    ("configs[4] N=2^28 distributed, NCCL all_to_all_single baseline, transposed-out", "huge", lambda: Huge(exchange="nccl"), 10)]
-        for label, name, make, nsteps in plan:
+            plan = [("configs[2] STFT, channels sharded (strong scaling)", "stft", STFT),
+                    ("configs[4] N=2^28 distributed, fused peer exchange, transposed-out", "huge", lambda: Huge(exchange="peer")),
+                    ("configs[4] N=2^28 distributed, fused peer exchange, natural order (second all-to-all fused)", "huge", lambda: Huge(natural=True, exchange="peer")),
+                    ("configs[4] N=2^28 distributed, NCCL all_to_all_single baseline, transposed-out", "huge", lambda: Huge(exchange="nccl"))]
+        for label, name, make in plan:
             try:
                 w = make()
-                rec = measure(w, name, ctx, nsteps, 3, not args.no_e2e, world == 1 and not args.no_cpu, 3.0)
+                rec = measure(w, name, ctx, args.steps, args.warmup, not args.no_e2e, world == 1 and not args.no_cpu, 3.0)
                 rec["baseline_config"] = label
                 release(w, torch)
             except Exception as e:  # a sub-record must not take the headline down

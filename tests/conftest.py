@@ -21,11 +21,26 @@ def oracle_mod():
     return o
 
 
+class Golden(dict):
+    """The arrays of several .npz files behind the interface of one (`.files`, `[name]`)."""
+
+    @property
+    def files(self):
+        return list(self)
+
+
 @pytest.fixture(scope="session")
 def golden():
+    """The reference's outputs written by tests/gen_golden.py, split into files of under 1 MB each."""
+    import glob
+
     import numpy as np
 
-    return np.load(os.path.join(ROOT, "tests", "golden", "reference_vectors.npz"))
+    g = Golden()
+    for path in sorted(glob.glob(os.path.join(ROOT, "tests", "golden", "reference_vectors*.npz"))):
+        with np.load(path) as f:
+            g.update((k, f[k]) for k in f.files)
+    return g
 
 
 @pytest.fixture(scope="session")

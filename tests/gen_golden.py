@@ -1,4 +1,4 @@
-"""Generates tests/golden/reference_vectors.npz by RUNNING THE UNMODIFIED REFERENCE
+"""Generates tests/golden/reference_vectors*.npz by RUNNING THE UNMODIFIED REFERENCE
 (oracle/_ref/libchowdsp_fft_ref.so, built by oracle/Makefile from /root/reference).
 
 The reference ships no golden vectors (its tests compare against pffft, which is not vendored,
@@ -44,9 +44,16 @@ def main():
         out[tag + "_bwd_unordered"] = bu
         out[tag + "_conv_acc_in"] = acc
         out[tag + "_conv_out"] = conv
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_vectors.npz")
-    np.savez_compressed(path, **out)
-    print(path, os.path.getsize(path), "bytes,", len(out), "arrays")
+    # one file per width for the largest size keeps every file under 1 MB
+    groups = {}
+    for key, arr in out.items():
+        N, W = key.split("_")[0][1:].split("w")
+        name = "reference_vectors.npz" if int(N) < 4096 else f"reference_vectors_{N}w{W}.npz"
+        groups.setdefault(name, {})[key] = arr
+    for name, arrays in groups.items():
+        path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name)
+        np.savez_compressed(path, **arrays)
+        print(path, os.path.getsize(path), "bytes,", len(arrays), "arrays")
 
 
 if __name__ == "__main__":

@@ -44,18 +44,18 @@ def test_reference_c_test_loop_on_the_gpu(tmp_path):
     assert "90 cases, 0 failures" in r.stdout and "Testing complete!" in r.stdout
 
 
-SAN = shutil.which("compute-sanitizer") or "/usr/local/cuda/bin/compute-sanitizer"
+# an installed but non-executable binary counts as absent
+SAN = shutil.which("compute-sanitizer", path=os.pathsep.join([os.environ.get("PATH", ""), "/usr/local/cuda/bin"]))
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("tool", ["memcheck", "racecheck"])
 def test_compute_sanitizer_clean(tmp_path, tool):
     """SURVEY.md §5 row 2 on the real hardware (the CPU emulator's TSan pass does not model the async proxy): one small
-    case per kernel family under compute-sanitizer; any report fails the test.  Logs are kept under gpurun_out/sanitizer/."""
-    if not os.path.exists(SAN):
-        pytest.skip("compute-sanitizer not installed")
-    out_dir = os.path.join(ROOT, "gpurun_out", "sanitizer")
-    os.makedirs(out_dir, exist_ok=True)
+    case per kernel family under compute-sanitizer; any report fails the test.  Logs are kept under the test's tmp_path."""
+    if SAN is None:
+        pytest.skip("compute-sanitizer not available")
+    out_dir = str(tmp_path)
     cmds = {"py": [SAN, "--tool", tool, "--error-exitcode", "9", "--print-limit", "20", "python", os.path.join(ROOT, "tools", "sanitizer_cases.py")]}
     if os.path.exists(REF_SO):
         cmds["c"] = [SAN, "--tool", tool, "--error-exitcode", "9", "--print-limit", "20", _build(tmp_path), "5", "16", REF_SO]
