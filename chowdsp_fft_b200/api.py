@@ -199,6 +199,36 @@ def fft_partitioned_convolve_step(setup: int, windows, window_stride: int, ir, i
                                                channels, partitions, block_index, scaling, _stream(stream)))
 
 
+# ---- streaming convolver with non-uniform partitions (chowdsp_fft_b200.h: fft_convolver_create ... fft_convolver_destroy) ----
+def fft_convolver_create(channels: int, block_size: int, ir, ir_length: int, ir_channel_stride: int, stream=None) -> int:
+    """Context that convolves `channels` signals with their IRs (ir + c*ir_channel_stride, 0 = one shared IR), block_size
+    samples per channel per fft_convolver_process call, with no added latency."""
+    ctx = C.c_void_p()
+    _check(lib().fft_convolver_create(channels, block_size, _addr(ir), ir_length, ir_channel_stride, _stream(stream), C.byref(ctx)))
+    return ctx.value
+
+
+def fft_convolver_process(ctx: int, input, input_stride: int, output, output_stride: int, stream=None) -> None:
+    _check(lib().fft_convolver_process(ctx, _addr(input), input_stride, _addr(output), output_stride, _stream(stream)))
+
+
+def fft_convolver_reset(ctx: int, stream=None) -> None:
+    _check(lib().fft_convolver_reset(ctx, _stream(stream)))
+
+
+def fft_convolver_segments(ctx: int) -> list[tuple[int, int]]:
+    """The context's schedule: [(block size, partitions)] per segment."""
+    n = lib().fft_convolver_segments(ctx, None, None, 0)
+    _check(min(n, 0))
+    blocks, parts = (C.c_int * n)(), (C.c_int * n)()
+    lib().fft_convolver_segments(ctx, blocks, parts, n)
+    return list(zip(blocks, parts))
+
+
+def fft_convolver_destroy(ctx: int) -> None:
+    _check(lib().fft_convolver_destroy(ctx))
+
+
 def set_tuning(key: str, value: int) -> None:
     """Benchmark/sweep hook (fft_b200_set_tuning)."""
     _check(lib().fft_b200_set_tuning(key.encode(), int(value)))

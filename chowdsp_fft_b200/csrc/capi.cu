@@ -2090,6 +2090,296 @@ CFB_API int fft_partitioned_convolve_step (void* setup, const float* windows, lo
     return e == cudaSuccess ? 0 : fail_cuda (e, "partitioned convolution kernel launch");
 }
 
+// ---- streaming convolver with non-uniform partitions (fft_convolver_*; schedule: conv_schedule in pconv_kernel.cuh) ----
+namespace
+{
+constexpr uint64_t kConvMagic = 0x434642434f4e5631ull; // "CFBCONV1"
+constexpr int kConvMaxSegments = 16;                   // B = 16 up to Bmax = 16384 needs 11
+constexpr int kConvMaxBlockDefault = 16384;            // the largest block of the fused step's real plans
+int g_conv_max_block = kConvMaxBlockDefault;           // tuning hook "convolver_max_block"
+
+struct ConvSegment
+{
+    int Bk = 0, P = 0;    // block size, partitions
+    long long start = 0;  // first tap (also the output delay for k >= 1)
+    Plan* plan = nullptr; // real plan of 2 Bk points
+    Tables tables;
+    float* ir = nullptr;  // [channels or 1][P][2 Bk] IR spectra, unordered layout
+    float* fdl = nullptr; // [channels][P][2 Bk] frequency-delay line
+};
+
+struct ConvCtx
+{
+    uint64_t magic;
+    int channels = 0, B = 0, Bmax = 0, nseg = 0, device = 0;
+    bool shared_ir = false;
+    ConvSegment seg[kConvMaxSegments];
+    float* hist = nullptr; // [channels][2 ring] mirrored input history, ring = 2 Bmax
+    float* acc = nullptr;  // [channels][ring] output accumulator
+    float* S = nullptr;    // [channels][2 Bmax] partial spectrum of a sliced last segment (P > 1), else null
+    long long ring = 0;
+    long long t = 0;       // calls since create / reset
+};
+
+ConvCtx* as_conv (void* ctx)
+{
+    auto* d = static_cast<ConvCtx*> (ctx);
+    if (d == nullptr || (reinterpret_cast<uintptr_t> (d) & 7) != 0 || d->magic != kConvMagic)
+    {
+        fail (chowdsp::fft::FFT_B200_EINVAL, "invalid convolver context %p", ctx);
+        return nullptr;
+    }
+    return d;
+}
+
+// block index for the fused step: the slot written is t % P and min(t + 1, P) partitions are summed, so a running count can be
+// folded to keep it in int range
+int fold_index (long long t, int P) { return t < P ? (int) t : (int) (t % P) + P; }
+
+void conv_free (ConvCtx* d)
+{
+    for (int k = 0; k < d->nseg; ++k)
+    {
+        (void) cudaFree (d->seg[k].ir);
+        (void) cudaFree (d->seg[k].fdl);
+        if (d->seg[k].plan != nullptr)
+            chowdsp::fft::fft_destroy_setup (d->seg[k].plan);
+    }
+    (void) cudaFree (d->hist);
+    (void) cudaFree (d->acc);
+    (void) cudaFree (d->S);
+    d->magic = 0;
+    delete d;
+}
+
+int conv_zero (ConvCtx* d, cudaStream_t st)
+{
+    const size_t C = (size_t) d->channels;
+    for (int k = 0; k < d->nseg; ++k)
+        CFB_CUDA (cudaMemsetAsync (d->seg[k].fdl, 0, sizeof (float) * C * (size_t) d->seg[k].P * 2 * (size_t) d->seg[k].Bk, st));
+    CFB_CUDA (cudaMemsetAsync (d->hist, 0, sizeof (float) * C * 2 * (size_t) d->ring, st));
+    CFB_CUDA (cudaMemsetAsync (d->acc, 0, sizeof (float) * C * (size_t) d->ring, st));
+    if (d->S != nullptr)
+        CFB_CUDA (cudaMemsetAsync (d->S, 0, sizeof (float) * C * 2 * (size_t) d->Bmax, st));
+    d->t = 0;
+    return 0;
+}
+
+int conv_build (ConvCtx* d, const float* ir, long long L, long long ir_stride, cudaStream_t st)
+{
+    int blocks[kConvMaxSegments];
+    long long parts[kConvMaxSegments], starts[kConvMaxSegments];
+    d->nseg = conv_schedule (d->B, L, d->Bmax, blocks, parts, starts, kConvMaxSegments);
+    if (d->nseg > kConvMaxSegments)
+        return fail (chowdsp::fft::FFT_B200_EINVAL, "fft_convolver_create: schedule of %d segments", d->nseg);
+    const size_t C = (size_t) d->channels, Cir = d->shared_ir ? 1 : C;
+    size_t tmp_floats = 0;
+    for (int k = 0; k < d->nseg; ++k)
+    {
+        if (parts[k] > (1 << 24))
+            return fail (chowdsp::fft::FFT_B200_EINVAL, "fft_convolver_create: ir_length %lld needs too many partitions", L);
+        ConvSegment& g = d->seg[k];
+        g.Bk = blocks[k];
+        g.P = (int) parts[k];
+        g.start = starts[k];
+        const size_t n = 2 * (size_t) g.Bk * (size_t) g.P;
+        tmp_floats = tmp_floats > Cir * n ? tmp_floats : Cir * n;
+        CFB_CUDA (cudaMalloc (&g.ir, sizeof (float) * Cir * n));
+        CFB_CUDA (cudaMalloc (&g.fdl, sizeof (float) * C * n));
+        g.plan = static_cast<Plan*> (chowdsp::fft::fft_new_setup (2 * g.Bk, chowdsp::fft::FFT_REAL, true));
+        if (g.plan == nullptr)
+            return chowdsp::fft::FFT_B200_ECUDA;
+        const int rc = plan_tables (g.plan, g.tables);
+        if (rc != 0)
+            return rc;
+    }
+    d->ring = 2LL * d->Bmax;
+    CFB_CUDA (cudaMalloc (&d->hist, sizeof (float) * C * 2 * (size_t) d->ring));
+    CFB_CUDA (cudaMalloc (&d->acc, sizeof (float) * C * (size_t) d->ring));
+    const ConvSegment& last = d->seg[d->nseg - 1];
+    if (d->nseg > 1 && last.P > 1)
+        CFB_CUDA (cudaMalloc (&d->S, sizeof (float) * C * 2 * (size_t) last.Bk));
+    int rc = conv_zero (d, st);
+    if (rc != 0)
+        return rc;
+    // IR spectra: zero-padded partitions [Bk taps | Bk zeros], forward-transformed in the plan's unordered layout
+    float* tmp = nullptr;
+    CFB_CUDA (cudaMalloc (&tmp, sizeof (float) * tmp_floats));
+    for (int k = 0; k < d->nseg && rc == 0; ++k)
+    {
+        const ConvSegment& g = d->seg[k];
+        const ConvIrArgs ga { ir, ir_stride, tmp, L, g.start, (int) Cir, g.P, g.Bk };
+        const cudaError_t e = launch_conv_ir_gather (ga, st);
+        if (e != cudaSuccess)
+            rc = fail_cuda (e, "IR partition gather");
+        else
+            rc = chowdsp::fft::fft_transform_batched (g.plan, tmp, g.ir, (int) Cir * g.P, 2LL * g.Bk, 2LL * g.Bk, chowdsp::fft::FFT_FORWARD, 0, st);
+    }
+    const cudaError_t es = cudaStreamSynchronize (st);
+    (void) cudaFree (tmp);
+    if (rc != 0)
+        return rc;
+    return es == cudaSuccess ? 0 : fail_cuda (es, "fft_convolver_create");
+}
+} // namespace
+
+CFB_API int fft_convolver_create (int channels, int block_size, const float* ir, long long ir_length, long long ir_channel_stride, void* stream, void** ctx_out)
+{
+    CFB_TRACE ("fft_convolver_create");
+    if (ctx_out == nullptr)
+        return fail (FFT_B200_EINVAL, "fft_convolver_create: null ctx_out");
+    *ctx_out = nullptr;
+    if (channels < 1 || block_size < 16 || block_size > kConvMaxBlockDefault || (block_size & (block_size - 1)) != 0 || ir == nullptr || ir_length < 1
+        || ir_channel_stride < 0 || (ir_channel_stride != 0 && ir_channel_stride < ir_length))
+        return fail (FFT_B200_EINVAL, "fft_convolver_create: bad arguments (channels >= 1, block_size a power of two in [16, 16384], ir_length >= 1, ir_channel_stride 0 or >= ir_length)");
+    if (misaligned (ir, 4))
+        return fail (FFT_B200_EINVAL, "fft_convolver_create: the IR must be 4-byte aligned");
+    if (! device_available())
+        return fail (FFT_B200_ENODEVICE, "no usable CUDA device: chowdsp_fft_b200 has no CPU fallback");
+    if (classify (ir).kind != Mem::Device)
+        return fail (FFT_B200_EINVAL, "fft_convolver_create needs a device pointer for the IR");
+    auto* d = new (std::nothrow) ConvCtx();
+    if (d == nullptr)
+        return fail (FFT_B200_ECUDA, "out of host memory");
+    d->magic = kConvMagic;
+    d->channels = channels;
+    d->B = block_size;
+    d->Bmax = g_conv_max_block > block_size ? g_conv_max_block : block_size;
+    d->shared_ir = ir_channel_stride == 0;
+    const cudaError_t e = cudaGetDevice (&d->device);
+    const int rc = e != cudaSuccess ? fail_cuda (e, "cudaGetDevice") : conv_build (d, ir, ir_length, ir_channel_stride, static_cast<cudaStream_t> (stream));
+    if (rc != 0)
+    {
+        (void) cudaStreamSynchronize (static_cast<cudaStream_t> (stream));
+        conv_free (d);
+        return rc;
+    }
+    *ctx_out = d;
+    return 0;
+}
+
+CFB_API int fft_convolver_process (void* ctx, const float* input, long long input_stride, float* output, long long output_stride, void* stream_)
+{
+    CFB_TRACE ("fft_convolver_process");
+    ConvCtx* d = as_conv (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    const int C = d->channels, B = d->B;
+    if (input == nullptr || output == nullptr)
+        return fail (FFT_B200_EINVAL, "fft_convolver_process: null buffer");
+    if (misaligned (input, 8, input_stride, C) || misaligned (output, 8, output_stride, C))
+        return fail (FFT_B200_EINVAL, "fft_convolver_process: input / output must be 8-byte aligned with even strides");
+    if (classify (input).kind != Mem::Device || classify (output).kind != Mem::Device)
+        return fail (FFT_B200_EINVAL, "fft_convolver_process needs device pointers");
+    int dev = 0;
+    CFB_CUDA (cudaGetDevice (&dev));
+    if (dev != d->device)
+        return fail (FFT_B200_EINVAL, "fft_convolver_process: the context lives on device %d, the current device is %d", d->device, dev);
+    cudaStream_t st = static_cast<cudaStream_t> (stream_);
+    const long long t = d->t, ring = d->ring;
+    const long long pos = (t * B) % ring, end = (pos + B) % ring; // ring position of this block and of the sample after it
+    cudaError_t e = launch_conv_input (ConvInputArgs { input, input_stride, d->hist, 2 * ring, C, B / 2, pos, ring }, st);
+    // segments k >= 1 fire when their block of Bk samples is complete and add their Bk results to the ring at [end, end + Bk):
+    // strictly after the block emitted now, and never wrapping (end is a multiple of Bk, ring = 2 Bmax)
+    for (int k = d->nseg - 1; k >= 1 && e == cudaSuccess; --k)
+    {
+        const ConvSegment& g = d->seg[k];
+        const int D = g.Bk / B;
+        const long long q = t / D; // the firing this call belongs to; it fires on the period's last call
+        const bool sliced = k == d->nseg - 1 && g.P > 1;
+        if (sliced)
+        {
+            const int s = (int) (t % D);
+            const PConvSliceArgs sa { g.ir, d->shared_ir ? 0 : (long long) g.P * 2 * g.Bk, g.fdl, (long long) g.P * 2 * g.Bk, d->S, 2LL * g.Bk,
+                                      C, g.P, 2 * g.Bk, g.plan->logW, (int) (q % g.P), s * (B / 4), B / 4 };
+            e = launch_pconv_slice (sa, st);
+        }
+        if ((t + 1) % D != 0 || e != cudaSuccess)
+            continue;
+        PConvArgs a {};
+        a.in = d->hist + ring + end - 2LL * g.Bk;
+        a.in_stride = 2 * ring;
+        a.ir = g.ir;
+        a.ir_ch_stride = d->shared_ir ? 0 : (long long) g.P * 2 * g.Bk;
+        a.fdl = g.fdl;
+        a.fdl_ch_stride = (long long) g.P * 2 * g.Bk;
+        a.out = d->acc + end;
+        a.out_stride = ring;
+        a.channels = C;
+        a.P = g.P;
+        a.t = fold_index (q, g.P);
+        a.scaling = 1.f / (float) (2 * g.Bk);
+        a.tw = g.tables.tw;
+        a.rtw = g.tables.rtw;
+        const PConvAcc x { nullptr, 0, d->S, 2LL * g.Bk };
+        e = launch_pconv_acc (g.plan->logM, g.plan->logW, PCONV_ADD, sliced, a, x, st);
+    }
+    if (e == cudaSuccess)
+    {
+        // segment 0 (block B, every call): output = its result + the ring's [pos, pos + B), which it clears
+        const ConvSegment& g = d->seg[0];
+        PConvArgs a {};
+        a.in = d->hist + ring + end - 2LL * B;
+        a.in_stride = 2 * ring;
+        a.ir = g.ir;
+        a.ir_ch_stride = d->shared_ir ? 0 : (long long) g.P * 2 * B;
+        a.fdl = g.fdl;
+        a.fdl_ch_stride = (long long) g.P * 2 * B;
+        a.out = output;
+        a.out_stride = output_stride;
+        a.channels = C;
+        a.P = g.P;
+        a.t = fold_index (t, g.P);
+        a.scaling = 1.f / (float) (2 * B);
+        a.tw = g.tables.tw;
+        a.rtw = g.tables.rtw;
+        if (d->nseg == 1) // uniform: nothing is ever added to the ring, the plain step writes the output
+            e = launch_pconv (g.plan->logM, g.plan->logW, a, st);
+        else
+            e = launch_pconv_acc (g.plan->logM, g.plan->logW, PCONV_EMIT, false, a, PConvAcc { d->acc + pos, ring, nullptr, 0 }, st);
+    }
+    note_kernel ("cfb::pconv_acc_kernel: streaming convolver, %d segments", d->nseg);
+    if (e != cudaSuccess)
+        return fail_cuda (e, "convolver launch");
+    d->t = t + 1;
+    return 0;
+}
+
+CFB_API int fft_convolver_reset (void* ctx, void* stream)
+{
+    CFB_TRACE ("fft_convolver_reset");
+    ConvCtx* d = as_conv (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    return conv_zero (d, static_cast<cudaStream_t> (stream));
+}
+
+CFB_API int fft_convolver_segments (void* ctx, int* block_sizes, int* partitions, int max_segments)
+{
+    ConvCtx* d = as_conv (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    for (int k = 0; k < d->nseg && k < max_segments; ++k)
+    {
+        if (block_sizes != nullptr)
+            block_sizes[k] = d->seg[k].Bk;
+        if (partitions != nullptr)
+            partitions[k] = d->seg[k].P;
+    }
+    return d->nseg;
+}
+
+CFB_API int fft_convolver_destroy (void* ctx)
+{
+    ConvCtx* d = as_conv (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    (void) cudaDeviceSynchronize(); // work queued on any stream may still use the buffers
+    conv_free (d);
+    (void) cudaGetLastError();
+    return 0;
+}
+
 CFB_API int fft_large_factors (void* setup, int* l1, int* l2, int* l3)
 {
     Plan* p = as_plan (setup);
@@ -2690,6 +2980,11 @@ CFB_API int fft_b200_set_tuning (const char* key, int value)
     if (key != nullptr && std::strcmp (key, "stft_pipe") == 0)
     {
         g_stft_pipe = value != 0;
+        return 0;
+    }
+    if (key != nullptr && std::strcmp (key, "convolver_max_block") == 0 && (value == -1 || (value >= 16 && value <= kConvMaxBlockDefault && (value & (value - 1)) == 0)))
+    {
+        g_conv_max_block = value == -1 ? kConvMaxBlockDefault : value;
         return 0;
     }
     if (key != nullptr && std::strcmp (key, "stft_union") == 0)

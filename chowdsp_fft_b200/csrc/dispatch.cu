@@ -10,6 +10,7 @@ namespace
 {
 std::atomic<unsigned long long> g_launches { 0 };
 }
+static int elementwise_grid (long long items, int threads);
 unsigned long long launch_count() { return g_launches.load (std::memory_order_relaxed); }
 void count_launch() { g_launches.fetch_add (1, std::memory_order_relaxed); }
 
@@ -36,6 +37,44 @@ cudaError_t launch_pconv (int logM, int logW, const PConvArgs& args, cudaStream_
 #undef X
         default: return cudaErrorInvalidValue;
     }
+}
+cudaError_t launch_pconv_acc (int logM, int logW, int mode, bool partial, const PConvArgs& args, const PConvAcc& acc, cudaStream_t stream)
+{
+    switch (logM)
+    {
+#define X(n) \
+    case n: return launch_pconv_acc_##n (logW, mode, partial, args, acc, stream);
+        CFB_FOR_SIZES (X)
+#undef X
+        default: return cudaErrorInvalidValue;
+    }
+}
+cudaError_t launch_pconv_slice (const PConvSliceArgs& args, cudaStream_t stream)
+{
+    const long long items = (long long) args.channels * args.pairs;
+    if (items <= 0)
+        return cudaSuccess;
+    pconv_slice_kernel<<<(unsigned) ((items + 255) / 256), 256, 0, stream>>> (args);
+    count_launch();
+    return cudaGetLastError();
+}
+cudaError_t launch_conv_input (const ConvInputArgs& args, cudaStream_t stream)
+{
+    const long long items = (long long) args.channels * args.half_block;
+    if (items <= 0)
+        return cudaSuccess;
+    conv_input_kernel<<<(unsigned) ((items + 255) / 256), 256, 0, stream>>> (args);
+    count_launch();
+    return cudaGetLastError();
+}
+cudaError_t launch_conv_ir_gather (const ConvIrArgs& args, cudaStream_t stream)
+{
+    const long long items = (long long) args.channels * args.P * 2 * args.Bk;
+    if (items <= 0)
+        return cudaSuccess;
+    conv_ir_gather_kernel<<<elementwise_grid (items, 256), 256, 0, stream>>> (args);
+    count_launch();
+    return cudaGetLastError();
 }
 cudaError_t launch_fft_juce (int logM, int kind, int radix, const FftArgs& args, cudaStream_t stream)
 {

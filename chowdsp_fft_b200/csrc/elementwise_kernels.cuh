@@ -1,7 +1,9 @@
 // Unordered-domain elementwise kernels: the frequency-domain multiply-accumulate behind
-// fft_convolve_unordered and the plain sum behind fft_accumulate.  Pure HBM streaming.
+// fft_convolve_unordered and the plain sum behind fft_accumulate, and the streaming convolver's helpers
+// (argument structs in pconv_kernel.cuh).  Pure HBM streaming.
 #pragma once
 #include "fft_kernels.cuh"
+#include "pconv_kernel.cuh"
 
 namespace cfb
 {
@@ -82,4 +84,62 @@ __global__ void __launch_bounds__ (256) juce_mirror_kernel (float* data, long lo
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// streaming convolver (fft_convolver_*)
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__ (256) pconv_slice_kernel (const PConvSliceArgs a)
+{
+    const long long item = (long long) blockIdx.x * blockDim.x + threadIdx.x;
+    if (item >= (long long) a.channels * a.pairs)
+        return;
+    const int c = (int) (item / a.pairs), pr = a.pair0 + (int) (item % a.pairs);
+    const int W = 1 << a.logW, lq = a.logW - 2;
+    const int off = ((pr >> lq) << (a.logW + 1)) + ((pr & ((1 << lq) - 1)) << 2);
+    const float* irc = a.ir + (long long) c * a.ir_ch_stride + off;
+    const float* fdlc = a.fdl + (long long) c * a.fdl_ch_stride + off;
+    float4 ar = make_float4 (0.f, 0.f, 0.f, 0.f), ai = ar;
+    float dc = 0.f, ny = 0.f;
+    int g = (a.q - 1 + a.P) % a.P; // slot of X_(q-1)
+    for (int p = 1; p < a.P; ++p)
+    {
+        const float* h = irc + (long long) p * a.N;
+        const float* xs = fdlc + (long long) g * a.N;
+        const float4 hr = ld_stream4 (h), hi = ld_stream4 (h + W), xr = ld_stream4 (xs), xi = ld_stream4 (xs + W);
+        dc = fmaf (xr.x, hr.x, dc);
+        ny = fmaf (xi.x, hi.x, ny);
+        cmac4 (ar, ai, xr, xi, hr, hi);
+        g = g == 0 ? a.P - 1 : g - 1;
+    }
+    if (pr == 0)
+    {
+        ar.x = dc;
+        ai.x = ny;
+    }
+    float* sc = a.S + (long long) c * a.s_stride + off;
+    *reinterpret_cast<float4*> (sc) = ar;
+    *reinterpret_cast<float4*> (sc + W) = ai;
+}
+
+__global__ void __launch_bounds__ (256) conv_input_kernel (const ConvInputArgs a)
+{
+    const long long item = (long long) blockIdx.x * blockDim.x + threadIdx.x;
+    if (item >= (long long) a.channels * a.half_block)
+        return;
+    const long long c = item / a.half_block, k = item % a.half_block;
+    const float2 v = *reinterpret_cast<const float2*> (a.in + c * a.in_stride + 2 * k);
+    float* h = a.hist + c * a.hist_stride + a.pos + 2 * k;
+    *reinterpret_cast<float2*> (h) = v;
+    *reinterpret_cast<float2*> (h + a.mirror) = v;
+}
+
+__global__ void __launch_bounds__ (256) conv_ir_gather_kernel (const ConvIrArgs a)
+{
+    const long long n2 = 2LL * a.Bk, total = (long long) a.channels * a.P * n2;
+    for (long long item = (long long) blockIdx.x * blockDim.x + threadIdx.x; item < total; item += (long long) gridDim.x * blockDim.x)
+    {
+        const long long i = item % n2, cp = item / n2, p = cp % a.P, c = cp / a.P;
+        const long long tap = a.start + p * a.Bk + i;
+        a.dst[item] = (i < a.Bk && tap < a.length) ? a.ir[c * a.ir_stride + tap] : 0.f;
+    }
+}
 } // namespace cfb

@@ -198,6 +198,48 @@ cudaError_t CFB_CAT (launch_pconv_, CFB_LOGM) (int logW, const PConvArgs& a, cud
 
 namespace
 {
+template <int LOGW, int MODE, bool PARTIAL>
+cudaError_t launch_pconv_acc_one (const PConvArgs& a, const PConvAcc& x, cudaStream_t stream)
+{
+    using PL = PConvLaunch<CFB_LOGM>;
+    auto kernel = pconv_acc_kernel<CFB_LOGM, LOGW, MODE, PARTIAL>;
+    constexpr int smem_bytes = PL::SMEM_BYTES;
+    if (smem_bytes > 48 * 1024)
+    {
+        const cudaError_t e = cudaFuncSetAttribute (kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+        if (e != cudaSuccess)
+            return e;
+    }
+    if (a.channels <= 0)
+        return cudaSuccess;
+    kernel<<<(unsigned) ((a.channels + PL::PER_CTA - 1) / PL::PER_CTA), PL::THREADS, smem_bytes, stream>>> (a, x);
+    count_launch();
+    return cudaGetLastError();
+}
+template <int LOGW>
+cudaError_t launch_pconv_acc_w (int mode, bool partial, const PConvArgs& a, const PConvAcc& x, cudaStream_t stream)
+{
+    if (mode == PCONV_EMIT && ! partial)
+        return launch_pconv_acc_one<LOGW, PCONV_EMIT, false> (a, x, stream);
+    if (mode == PCONV_ADD)
+        return partial ? launch_pconv_acc_one<LOGW, PCONV_ADD, true> (a, x, stream) : launch_pconv_acc_one<LOGW, PCONV_ADD, false> (a, x, stream);
+    return cudaErrorInvalidValue;
+}
+} // namespace
+
+cudaError_t CFB_CAT (launch_pconv_acc_, CFB_LOGM) (int logW, int mode, bool partial, const PConvArgs& a, const PConvAcc& x, cudaStream_t stream)
+{
+    if (logW == 2)
+        return launch_pconv_acc_w<2> (mode, partial, a, x, stream);
+#if CFB_LOGM >= 6
+    if (logW == 3)
+        return launch_pconv_acc_w<3> (mode, partial, a, x, stream);
+#endif
+    return cudaErrorInvalidValue;
+}
+
+namespace
+{
 template <int R, int LOGW, bool UNION>
 cudaError_t launch_stft_one (const FftArgs& a, cudaStream_t stream)
 {

@@ -55,8 +55,29 @@ struct PConvLaunch
     static constexpr int SMEM_BYTES = PER_CTA * G::SMEM_F2_UNORD * 8;
 };
 
-template <int LOGM, int LOGW>
-FFT_HD void pconv_body (const PConvArgs& a)
+// Output modes of the fused step (template parameter of pconv_body; PCONV_WRITE is the plain block step above).  The streaming
+// convolver (fft_convolver_*) sums segments of different block sizes in a per-channel accumulator ring:
+//   PCONV_ADD   out[n] += y[n]                       (a segment's delayed contribution, strictly in the future of the ring)
+//   PCONV_EMIT  out[n]  = y[n] + acc[n], acc[n] = 0  (the block being emitted; frees that ring region for later additions)
+// PARTIAL: the accumulator starts from a precomputed partial spectrum S (sum of the older partitions, pconv_slice_kernel) and
+// only the newest spectrum X_t (p = 0) is multiplied in here; slot t % P of the delay line is still written.
+enum PConvMode
+{
+    PCONV_WRITE = 0,
+    PCONV_ADD = 1,
+    PCONV_EMIT = 2
+};
+
+struct PConvAcc
+{
+    float* acc;         // PCONV_EMIT: channel c's ring region at acc + c * acc_stride (N/2 samples)
+    long long acc_stride;
+    const float* S;     // PARTIAL: channel c's partial spectrum at S + c * s_stride (N floats, unordered, unscaled)
+    long long s_stride;
+};
+
+template <int LOGM, int LOGW, int MODE = PCONV_WRITE, bool PARTIAL = false>
+FFT_HD void pconv_body (const PConvArgs& a, const PConvAcc& x = PConvAcc {})
 {
     constexpr int R = 16;
     using G = Geo<LOGM, R>;
@@ -92,16 +113,25 @@ FFT_HD void pconv_body (const PConvArgs& a)
             *reinterpret_cast<float4*> (slot + off[i]) = xr[i];     // delay-line write (linear across the channel's threads)
             *reinterpret_cast<float4*> (slot + off[i] + W) = xi[i];
         }
-        ar[i] = make_float4 (0.f, 0.f, 0.f, 0.f);
-        ai[i] = make_float4 (0.f, 0.f, 0.f, 0.f);
+        if constexpr (PARTIAL)
+        {
+            const float* sc = x.S + (long long) c * x.s_stride;
+            ar[i] = ld_stream4 (sc + off[i]);
+            ai[i] = ld_stream4 (sc + off[i] + W);
+        }
+        else
+        {
+            ar[i] = make_float4 (0.f, 0.f, 0.f, 0.f);
+            ai[i] = make_float4 (0.f, 0.f, 0.f, 0.f);
+        }
     }
 
     // 3. frequency-domain multiply-accumulate over the partitions; DC / Nyquist (float slots 0 and W of a
     //    real spectrum, lane 0 of this CTA's first pair) are two independent REAL products
-    float dc = 0.f, ny = 0.f;
+    float dc = PARTIAL ? ar[0].x : 0.f, ny = PARTIAL ? ai[0].x : 0.f;
     const float* irc = a.ir + (long long) c * a.ir_ch_stride;
     const float* fdlc = a.fdl + (long long) c * a.fdl_ch_stride;
-    const int np = a.t + 1 < a.P ? a.t + 1 : a.P;
+    const int np = PARTIAL ? 1 : (a.t + 1 < a.P ? a.t + 1 : a.P);
     for (int p = 0; p < np; ++p)
     {
         const float* h = irc + (long long) p * N;
@@ -148,7 +178,30 @@ FFT_HD void pconv_body (const PConvArgs& a)
 
     // 5. inverse transform; only the last N/2 samples are valid in overlap-save and only they are stored
     float* outc = a.out + (long long) c * a.out_stride - M; // sample n >= M lands at out[n - M]
-    fft_core<LOGM, R, C2R, LOGW, true, false, true> (nullptr, outc, active, j, smem, a.tw, a.rtw);
+    if constexpr (MODE == PCONV_WRITE)
+        fft_core<LOGM, R, C2R, LOGW, true, false, true> (nullptr, outc, active, j, smem, a.tw, a.rtw);
+    else
+    {
+        // the same inverse transform with the result handed back in registers (element j + m T in v[m]); the store adds
+        float2 v[R];
+        fft_core<LOGM, R, C2R, LOGW, true, false, true, 0, NoHook, true> (nullptr, nullptr, active, j, smem, a.tw, a.rtw, nullptr, nullptr, NoHook(), v);
+        if (active)
+        {
+            float2* o2 = reinterpret_cast<float2*> (outc) + j;
+            float2* acc2 = MODE == PCONV_EMIT ? reinterpret_cast<float2*> (x.acc + (long long) c * x.acc_stride - M) + j : nullptr;
+#pragma unroll
+            for (int m = R / 2; m < R; ++m)
+            {
+                if constexpr (MODE == PCONV_ADD)
+                    o2[m * T] = f2_add (o2[m * T], v[m]);
+                else
+                {
+                    o2[m * T] = f2_add (v[m], acc2[m * T]);
+                    acc2[m * T] = make_float2 (0.f, 0.f);
+                }
+            }
+        }
+    }
 }
 
 template <int LOGM, int LOGW>
@@ -156,4 +209,95 @@ __global__ void __launch_bounds__ (PConvLaunch<LOGM>::THREADS, (PConvLaunch<LOGM
 {
     pconv_body<LOGM, LOGW> (a);
 }
+
+// the accumulating modes (streaming convolver): one instance per (MODE, PARTIAL) in use
+template <int LOGM, int LOGW, int MODE, bool PARTIAL>
+__global__ void __launch_bounds__ (PConvLaunch<LOGM>::THREADS, (PConvLaunch<LOGM>::THREADS <= 256 ? 2 : 1)) pconv_acc_kernel (const PConvArgs a, const PConvAcc x)
+{
+    pconv_body<LOGM, LOGW, MODE, PARTIAL> (a, x);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Sliced tail multiply-accumulate of the streaming convolver (pconv_slice_kernel, elementwise_kernels.cuh): the part of a P-partition segment's spectral sum that does not
+// depend on the newest block,  S = sum_{p=1}^{P-1} X_(q-p) * H_p  (X_g in delay-line slot g % P, unscaled), for one slice of
+// the spectrum -- pairs [pair0, pair0 + pairs), a pair being 4 re lanes at float offset off and their 4 im lanes at off + W.
+// Spread over the small steps between two firings of the segment, every bin of S is written once per period and the firing
+// itself (pconv_acc_kernel<.., PARTIAL>) only multiplies X_q * H_0.  Same products and real DC / Nyquist lanes as pconv_body.
+struct PConvSliceArgs
+{
+    const float* ir;   // partition p of channel c: ir + c * ir_ch_stride + p * N
+    long long ir_ch_stride;
+    const float* fdl;  // slot g of channel c: fdl + c * fdl_ch_stride + g * N
+    long long fdl_ch_stride;
+    float* S;          // channel c's partial spectrum: S + c * s_stride
+    long long s_stride;
+    int channels;
+    int P;
+    int N;
+    int logW;
+    int q;             // the firing S is for
+    int pair0, pairs;
+};
+
+// Non-uniform partition schedule of the streaming convolver (host code; the emulator driver exposes it to the tests).  For
+// block B, IR length L and largest block Bmax (>= B):  segment 0 has block B and 2 partitions (taps [0, 2B)); segment k >= 1
+// has block Bk = 2^k B and one partition (taps [Bk, 2 Bk), output delay Bk) until Bk = Bmax, which takes the rest of the IR
+// in ceil((L - Bmax) / Bmax) partitions; the schedule stops as soon as the IR is covered.  L <= 2B or Bmax == B: one uniform
+// segment of ceil(L / B) partitions.  Writes up to max_segments (block, partitions, first tap) entries; returns the count.
+inline int conv_schedule (int B, long long L, int Bmax, int* block, long long* parts, long long* start, int max_segments)
+{
+    int n = 0;
+    auto put = [&] (int bk, long long p, long long s0)
+    {
+        if (n < max_segments)
+        {
+            block[n] = bk;
+            parts[n] = p;
+            start[n] = s0;
+        }
+        ++n;
+    };
+    if (L <= 2LL * B || Bmax <= B)
+    {
+        put (B, (L + B - 1) / B, 0);
+        return n;
+    }
+    put (B, 2, 0);
+    for (long long bk = 2LL * B; bk < L; bk *= 2)
+    {
+        if (bk >= Bmax)
+        {
+            put ((int) bk, (L - bk + bk - 1) / bk, bk);
+            break;
+        }
+        put ((int) bk, 1, bk);
+    }
+    return n;
+}
+
+// The convolver's input history (conv_input_kernel, elementwise_kernels.cuh): each channel's new block of B samples is written at pos and again at pos + mirror of a
+// mirrored ring (2 x mirror floats per channel), so that every window -- the last 2 B_k samples -- is one contiguous span.
+struct ConvInputArgs
+{
+    const float* in;   // channel c's block: in + c * in_stride, B samples (8-byte aligned, even stride)
+    long long in_stride;
+    float* hist;       // channel c's ring: hist + c * hist_stride
+    long long hist_stride;
+    int channels;
+    int half_block;    // B / 2 float2 per channel
+    long long pos, mirror;
+};
+
+// IR preparation (conv_ir_gather_kernel, elementwise_kernels.cuh; at context creation, not on the streaming path): partition p of channel c of a segment with block Bk,
+// starting at tap `start`, as the zero-padded window [Bk taps | Bk zeros] at dst + (c * P + p) * 2 Bk; taps past `length`
+// are zeros.  The forward transform of these windows is done by the ordinary batched transform.
+struct ConvIrArgs
+{
+    const float* ir;
+    long long ir_stride;
+    float* dst;
+    long long length, start;
+    int channels, P, Bk;
+};
+
 } // namespace cfb

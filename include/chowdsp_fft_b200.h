@@ -96,6 +96,29 @@ int fft_convolve_unordered_batched (void* setup, const float* dft_a, const float
    (test/test.cpp:214-218 shows the pattern), in one launch.  Device pointers only; stream-ordered. */
 int fft_partitioned_convolve_step (void* setup, const float* windows, long long window_stride, const float* ir, long long ir_channel_stride, float* fdl, long long fdl_channel_stride, float* output, long long output_stride, int channels, int partitions, int block_index, float scaling, void* stream);
 
+/* Streaming convolution of `channels` real signals with long impulse responses at a small block size: a stateful context
+   that takes B = block_size new samples per channel per call and returns B convolved samples per channel, with no added
+   latency.  Call t (counted from create or reset) reads x_c[tB .. (t+1)B) at input + c*input_stride and writes
+   y_c[tB .. (t+1)B) at output + c*output_stride, where y_c[n] = sum_{m < ir_length} h_c[m] x_c[n-m] (the true linear
+   convolution, normalised; the input before the first call is silence).  h_c is at ir + c*ir_channel_stride;
+   ir_channel_stride = 0 shares one IR across all channels (stored and transformed once).
+   The IR is split non-uniformly (fft_convolver_segments reports the schedule): segment 0 has block B and two partitions,
+   segment k >= 1 block 2^k B and one partition, up to the largest block Bmax (16384, tuning hook "convolver_max_block"),
+   which takes the rest of the IR; small blocks keep the latency, large ones cut the memory traffic per sample.
+     fft_convolver_create    allocates and zeroes the state and transforms the IR partitions (synchronous on `stream`);
+                             16 <= block_size <= 16384, a power of two; ir_length >= 1; ir_channel_stride 0 or >= ir_length
+     fft_convolver_process   one block per channel; input / output 8-byte aligned with even strides; stream-ordered
+     fft_convolver_reset     back to silence (the IR is kept); stream-ordered
+     fft_convolver_segments  up to max_segments (block size, partitions) pairs (either array may be NULL); returns the count
+     fft_convolver_destroy   waits for the device, then frees the context
+   Device pointers only.  Calls on one context must be ordered on one stream, on the device that was current at create,
+   and a context must not be used from two threads at the same time. */
+int fft_convolver_create (int channels, int block_size, const float* ir, long long ir_length, long long ir_channel_stride, void* stream, void** ctx_out);
+int fft_convolver_process (void* ctx, const float* input, long long input_stride, float* output, long long output_stride, void* stream);
+int fft_convolver_reset (void* ctx, void* stream);
+int fft_convolver_segments (void* ctx, int* block_sizes, int* partitions, int max_segments);
+int fft_convolver_destroy (void* ctx);
+
 /* Distributed four-step transform of ONE complex transform of N = 2^n >= 2^21 points over `world` GPUs
    (one process per GPU): the three LOCAL phases; the exchange between phase 0 and phase 1 is an
    all-to-all of equal contiguous chunks (NCCL, or peer stores, see fft_dist_phase0_peer).
@@ -191,7 +214,9 @@ void fft_b200_clear_error (void);
      "mixq"         1 = sizes Q 2^p with Q in {3, 5, 9, 15} run in mixq_kernel (default), 0 = always the generic mixed-radix kernel
      "zero_copy_kb" pinned (device-mapped) host buffers up to this many KiB are transformed in place over PCIe by the kernel's own
                     loads / stores instead of being staged through device memory (default 256)
-     "pf_ahead"     L2 prefetch distance of the single-kernel transforms in CTAs (default 0 = off) */
+     "pf_ahead"     L2 prefetch distance of the single-kernel transforms in CTAs (default 0 = off)
+     "convolver_max_block"  largest block of the streaming convolver's schedule for contexts created afterwards: a power of two
+                    in [16, 16384] (default 16384; a value <= block_size makes the schedule uniform) */
 int fft_b200_set_tuning (const char* key, int value);
 
 /* Number of CUDA kernels this library has launched in this process (all threads). */
