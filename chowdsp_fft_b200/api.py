@@ -212,6 +212,12 @@ def fft_convolver_process(ctx: int, input, input_stride: int, output, output_str
     _check(lib().fft_convolver_process(ctx, _addr(input), input_stride, _addr(output), output_stride, _stream(stream)))
 
 
+def fft_convolver_set_ir(ctx: int, ir, ir_length: int, ir_channel_stride: int, fade_blocks: int = 0, stream=None) -> None:
+    """Replace the context's IR while it runs: instantly (fade_blocks = 0) or with a linear crossfade over fade_blocks calls,
+    keeping the reverb tail of the input already played (see chowdsp_fft_b200.h)."""
+    _check(lib().fft_convolver_set_ir(ctx, _addr(ir), ir_length, ir_channel_stride, fade_blocks, _stream(stream)))
+
+
 def fft_convolver_reset(ctx: int, stream=None) -> None:
     _check(lib().fft_convolver_reset(ctx, _stream(stream)))
 

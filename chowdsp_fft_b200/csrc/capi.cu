@@ -2104,8 +2104,15 @@ struct ConvSegment
     long long start = 0;  // first tap (also the output delay for k >= 1)
     Plan* plan = nullptr; // real plan of 2 Bk points
     Tables tables;
-    float* ir = nullptr;  // [channels or 1][P][2 Bk] IR spectra, unordered layout
     float* fdl = nullptr; // [channels][P][2 Bk] frequency-delay line
+};
+
+// the state that depends on the IR; the input history and the delay lines depend on the input only and are shared by both banks
+struct ConvBank
+{
+    float* ir[kConvMaxSegments] = {}; // per segment [channels or 1][P][2 Bk] IR spectra, unordered layout
+    float* acc = nullptr;             // [channels][ring] output accumulator
+    float* S = nullptr;               // [channels][2 Bmax] partial spectrum of a sliced last segment (P > 1), else null
 };
 
 struct ConvCtx
@@ -2113,12 +2120,17 @@ struct ConvCtx
     uint64_t magic;
     int channels = 0, B = 0, Bmax = 0, nseg = 0, device = 0;
     bool shared_ir = false;
+    long long L = 0;       // IR length at create: the schedule covers it, and later IRs may not be longer
     ConvSegment seg[kConvMaxSegments];
+    ConvBank bank[2];      // bank[cur] holds the IR in use; bank[1 - cur] takes the next one (allocated by the first set_ir)
+    int cur = 0;
+    float* scratch = nullptr; // set_ir's IR partition gather buffer (scratch_floats), allocated with the second bank
+    size_t scratch_floats = 0;
     float* hist = nullptr; // [channels][2 ring] mirrored input history, ring = 2 Bmax
-    float* acc = nullptr;  // [channels][ring] output accumulator
-    float* S = nullptr;    // [channels][2 Bmax] partial spectrum of a sliced last segment (P > 1), else null
     long long ring = 0;
     long long t = 0;       // calls since create / reset
+    int fade = 0;          // > 0: calls [fade_t0, fade_t0 + fade) crossfade from bank[cur] to bank[1 - cur]
+    long long fade_t0 = 0;
 };
 
 ConvCtx* as_conv (void* ctx)
@@ -2136,18 +2148,42 @@ ConvCtx* as_conv (void* ctx)
 // folded to keep it in int range
 int fold_index (long long t, int P) { return t < P ? (int) t : (int) (t % P) + P; }
 
+void conv_bank_free (ConvBank& b)
+{
+    for (float*& p : b.ir)
+    {
+        (void) cudaFree (p);
+        p = nullptr;
+    }
+    (void) cudaFree (b.acc);
+    (void) cudaFree (b.S);
+    b.acc = b.S = nullptr;
+}
+
+int conv_bank_alloc (const ConvCtx* d, ConvBank& b)
+{
+    const size_t C = (size_t) d->channels, Cir = d->shared_ir ? 1 : C;
+    for (int k = 0; k < d->nseg; ++k)
+        CFB_CUDA (cudaMalloc (&b.ir[k], sizeof (float) * Cir * 2 * (size_t) d->seg[k].Bk * (size_t) d->seg[k].P));
+    CFB_CUDA (cudaMalloc (&b.acc, sizeof (float) * C * (size_t) d->ring));
+    const ConvSegment& last = d->seg[d->nseg - 1];
+    if (d->nseg > 1 && last.P > 1)
+        CFB_CUDA (cudaMalloc (&b.S, sizeof (float) * C * 2 * (size_t) last.Bk));
+    return 0;
+}
+
 void conv_free (ConvCtx* d)
 {
     for (int k = 0; k < d->nseg; ++k)
     {
-        (void) cudaFree (d->seg[k].ir);
         (void) cudaFree (d->seg[k].fdl);
         if (d->seg[k].plan != nullptr)
             chowdsp::fft::fft_destroy_setup (d->seg[k].plan);
     }
+    conv_bank_free (d->bank[0]);
+    conv_bank_free (d->bank[1]);
+    (void) cudaFree (d->scratch);
     (void) cudaFree (d->hist);
-    (void) cudaFree (d->acc);
-    (void) cudaFree (d->S);
     d->magic = 0;
     delete d;
 }
@@ -2155,13 +2191,33 @@ void conv_free (ConvCtx* d)
 int conv_zero (ConvCtx* d, cudaStream_t st)
 {
     const size_t C = (size_t) d->channels;
+    const ConvBank& b = d->bank[d->cur];
     for (int k = 0; k < d->nseg; ++k)
         CFB_CUDA (cudaMemsetAsync (d->seg[k].fdl, 0, sizeof (float) * C * (size_t) d->seg[k].P * 2 * (size_t) d->seg[k].Bk, st));
     CFB_CUDA (cudaMemsetAsync (d->hist, 0, sizeof (float) * C * 2 * (size_t) d->ring, st));
-    CFB_CUDA (cudaMemsetAsync (d->acc, 0, sizeof (float) * C * (size_t) d->ring, st));
-    if (d->S != nullptr)
-        CFB_CUDA (cudaMemsetAsync (d->S, 0, sizeof (float) * C * 2 * (size_t) d->Bmax, st));
+    CFB_CUDA (cudaMemsetAsync (b.acc, 0, sizeof (float) * C * (size_t) d->ring, st));
+    if (b.S != nullptr)
+        CFB_CUDA (cudaMemsetAsync (b.S, 0, sizeof (float) * C * 2 * (size_t) d->Bmax, st));
     d->t = 0;
+    return 0;
+}
+
+// IR spectra of bank b: zero-padded partitions [Bk taps | Bk zeros] gathered into tmp, forward-transformed in the plan's
+// unordered layout.  create and set_ir run this same sequence, so equal IRs give bitwise equal spectra.
+int conv_prepare_ir (const ConvCtx* d, ConvBank& b, const float* ir, long long L, long long ir_stride, float* tmp, cudaStream_t st)
+{
+    const int Cir = d->shared_ir ? 1 : d->channels;
+    for (int k = 0; k < d->nseg; ++k)
+    {
+        const ConvSegment& g = d->seg[k];
+        const ConvIrArgs ga { ir, ir_stride, tmp, L, g.start, Cir, g.P, g.Bk };
+        const cudaError_t e = launch_conv_ir_gather (ga, st);
+        if (e != cudaSuccess)
+            return fail_cuda (e, "IR partition gather");
+        const int rc = chowdsp::fft::fft_transform_batched (g.plan, tmp, b.ir[k], Cir * g.P, 2LL * g.Bk, 2LL * g.Bk, chowdsp::fft::FFT_FORWARD, 0, st);
+        if (rc != 0)
+            return rc;
+    }
     return 0;
 }
 
@@ -2172,8 +2228,8 @@ int conv_build (ConvCtx* d, const float* ir, long long L, long long ir_stride, c
     d->nseg = conv_schedule (d->B, L, d->Bmax, blocks, parts, starts, kConvMaxSegments);
     if (d->nseg > kConvMaxSegments)
         return fail (chowdsp::fft::FFT_B200_EINVAL, "fft_convolver_create: schedule of %d segments", d->nseg);
+    d->L = L;
     const size_t C = (size_t) d->channels, Cir = d->shared_ir ? 1 : C;
-    size_t tmp_floats = 0;
     for (int k = 0; k < d->nseg; ++k)
     {
         if (parts[k] > (1 << 24))
@@ -2183,8 +2239,7 @@ int conv_build (ConvCtx* d, const float* ir, long long L, long long ir_stride, c
         g.P = (int) parts[k];
         g.start = starts[k];
         const size_t n = 2 * (size_t) g.Bk * (size_t) g.P;
-        tmp_floats = tmp_floats > Cir * n ? tmp_floats : Cir * n;
-        CFB_CUDA (cudaMalloc (&g.ir, sizeof (float) * Cir * n));
+        d->scratch_floats = d->scratch_floats > Cir * n ? d->scratch_floats : Cir * n;
         CFB_CUDA (cudaMalloc (&g.fdl, sizeof (float) * C * n));
         g.plan = static_cast<Plan*> (chowdsp::fft::fft_new_setup (2 * g.Bk, chowdsp::fft::FFT_REAL, true));
         if (g.plan == nullptr)
@@ -2195,31 +2250,55 @@ int conv_build (ConvCtx* d, const float* ir, long long L, long long ir_stride, c
     }
     d->ring = 2LL * d->Bmax;
     CFB_CUDA (cudaMalloc (&d->hist, sizeof (float) * C * 2 * (size_t) d->ring));
-    CFB_CUDA (cudaMalloc (&d->acc, sizeof (float) * C * (size_t) d->ring));
-    const ConvSegment& last = d->seg[d->nseg - 1];
-    if (d->nseg > 1 && last.P > 1)
-        CFB_CUDA (cudaMalloc (&d->S, sizeof (float) * C * 2 * (size_t) last.Bk));
-    int rc = conv_zero (d, st);
+    int rc = conv_bank_alloc (d, d->bank[0]);
+    if (rc == 0)
+        rc = conv_zero (d, st);
     if (rc != 0)
         return rc;
-    // IR spectra: zero-padded partitions [Bk taps | Bk zeros], forward-transformed in the plan's unordered layout
     float* tmp = nullptr;
-    CFB_CUDA (cudaMalloc (&tmp, sizeof (float) * tmp_floats));
-    for (int k = 0; k < d->nseg && rc == 0; ++k)
-    {
-        const ConvSegment& g = d->seg[k];
-        const ConvIrArgs ga { ir, ir_stride, tmp, L, g.start, (int) Cir, g.P, g.Bk };
-        const cudaError_t e = launch_conv_ir_gather (ga, st);
-        if (e != cudaSuccess)
-            rc = fail_cuda (e, "IR partition gather");
-        else
-            rc = chowdsp::fft::fft_transform_batched (g.plan, tmp, g.ir, (int) Cir * g.P, 2LL * g.Bk, 2LL * g.Bk, chowdsp::fft::FFT_FORWARD, 0, st);
-    }
+    CFB_CUDA (cudaMalloc (&tmp, sizeof (float) * d->scratch_floats));
+    rc = conv_prepare_ir (d, d->bank[0], ir, L, ir_stride, tmp, st);
     const cudaError_t es = cudaStreamSynchronize (st);
     (void) cudaFree (tmp);
     if (rc != 0)
         return rc;
     return es == cudaSuccess ? 0 : fail_cuda (es, "fft_convolver_create");
+}
+
+long long conv_ir_stride (const ConvCtx* d, const ConvSegment& g) { return d->shared_ir ? 0 : (long long) g.P * 2 * g.Bk; }
+
+// slice [pair0, pair0 + pairs) of bank b's partial spectrum S for firing q of the last segment k
+cudaError_t conv_slice (const ConvCtx* d, const ConvBank& b, int k, long long q, int pair0, int pairs, cudaStream_t st)
+{
+    const ConvSegment& g = d->seg[k];
+    const PConvSliceArgs sa { b.ir[k], conv_ir_stride (d, g), g.fdl, (long long) g.P * 2 * g.Bk, b.S, 2LL * g.Bk,
+                              d->channels, g.P, 2 * g.Bk, g.plan->logW, (int) (q % g.P), pair0, pairs };
+    return launch_pconv_slice (sa, st);
+}
+
+// firing q of segment k >= 1 with bank b: adds its Bk results into the bank's ring at [end, end + Bk).  from_fdl takes X_q from
+// the delay line (written by the current bank's firing, or by the firing being re-run) instead of transforming the window.
+cudaError_t conv_fire (const ConvCtx* d, const ConvBank& b, int k, long long q, long long end, bool from_fdl, cudaStream_t st)
+{
+    const ConvSegment& g = d->seg[k];
+    const bool sliced = k == d->nseg - 1 && g.P > 1;
+    PConvArgs a {};
+    a.in = d->hist + d->ring + end - 2LL * g.Bk;
+    a.in_stride = 2 * d->ring;
+    a.ir = b.ir[k];
+    a.ir_ch_stride = conv_ir_stride (d, g);
+    a.fdl = g.fdl;
+    a.fdl_ch_stride = (long long) g.P * 2 * g.Bk;
+    a.out = b.acc + end;
+    a.out_stride = d->ring;
+    a.channels = d->channels;
+    a.P = g.P;
+    a.t = fold_index (q, g.P);
+    a.scaling = 1.f / (float) (2 * g.Bk);
+    a.tw = g.tables.tw;
+    a.rtw = g.tables.rtw;
+    const PConvAcc x { nullptr, 0, b.S, 2LL * g.Bk };
+    return launch_pconv_acc (g.plan->logM, g.plan->logW, PCONV_ADD, sliced, from_fdl, a, x, st);
 }
 } // namespace
 
@@ -2278,6 +2357,8 @@ CFB_API int fft_convolver_process (void* ctx, const float* input, long long inpu
     cudaStream_t st = static_cast<cudaStream_t> (stream_);
     const long long t = d->t, ring = d->ring;
     const long long pos = (t * B) % ring, end = (pos + B) % ring; // ring position of this block and of the sample after it
+    // during a crossfade the next bank runs every step after the current one, on the delay-line spectra the current one stores
+    const int banks = d->fade > 0 ? 2 : 1;
     cudaError_t e = launch_conv_input (ConvInputArgs { input, input_stride, d->hist, 2 * ring, C, B / 2, pos, ring }, st);
     // segments k >= 1 fire when their block of Bk samples is complete and add their Bk results to the ring at [end, end + Bk):
     // strictly after the block emitted now, and never wrapping (end is a multiple of Bk, ring = 2 Bmax)
@@ -2287,32 +2368,14 @@ CFB_API int fft_convolver_process (void* ctx, const float* input, long long inpu
         const int D = g.Bk / B;
         const long long q = t / D; // the firing this call belongs to; it fires on the period's last call
         const bool sliced = k == d->nseg - 1 && g.P > 1;
-        if (sliced)
+        for (int i = 0; i < banks && e == cudaSuccess; ++i)
         {
-            const int s = (int) (t % D);
-            const PConvSliceArgs sa { g.ir, d->shared_ir ? 0 : (long long) g.P * 2 * g.Bk, g.fdl, (long long) g.P * 2 * g.Bk, d->S, 2LL * g.Bk,
-                                      C, g.P, 2 * g.Bk, g.plan->logW, (int) (q % g.P), s * (B / 4), B / 4 };
-            e = launch_pconv_slice (sa, st);
+            const ConvBank& b = d->bank[d->cur ^ i];
+            if (sliced)
+                e = conv_slice (d, b, k, q, (int) (t % D) * (B / 4), B / 4, st);
+            if ((t + 1) % D == 0 && e == cudaSuccess)
+                e = conv_fire (d, b, k, q, end, i == 1, st);
         }
-        if ((t + 1) % D != 0 || e != cudaSuccess)
-            continue;
-        PConvArgs a {};
-        a.in = d->hist + ring + end - 2LL * g.Bk;
-        a.in_stride = 2 * ring;
-        a.ir = g.ir;
-        a.ir_ch_stride = d->shared_ir ? 0 : (long long) g.P * 2 * g.Bk;
-        a.fdl = g.fdl;
-        a.fdl_ch_stride = (long long) g.P * 2 * g.Bk;
-        a.out = d->acc + end;
-        a.out_stride = ring;
-        a.channels = C;
-        a.P = g.P;
-        a.t = fold_index (q, g.P);
-        a.scaling = 1.f / (float) (2 * g.Bk);
-        a.tw = g.tables.tw;
-        a.rtw = g.tables.rtw;
-        const PConvAcc x { nullptr, 0, d->S, 2LL * g.Bk };
-        e = launch_pconv_acc (g.plan->logM, g.plan->logW, PCONV_ADD, sliced, a, x, st);
     }
     if (e == cudaSuccess)
     {
@@ -2321,8 +2384,8 @@ CFB_API int fft_convolver_process (void* ctx, const float* input, long long inpu
         PConvArgs a {};
         a.in = d->hist + ring + end - 2LL * B;
         a.in_stride = 2 * ring;
-        a.ir = g.ir;
-        a.ir_ch_stride = d->shared_ir ? 0 : (long long) g.P * 2 * B;
+        a.ir = d->bank[d->cur].ir[0];
+        a.ir_ch_stride = conv_ir_stride (d, g);
         a.fdl = g.fdl;
         a.fdl_ch_stride = (long long) g.P * 2 * B;
         a.out = output;
@@ -2336,12 +2399,108 @@ CFB_API int fft_convolver_process (void* ctx, const float* input, long long inpu
         if (d->nseg == 1) // uniform: nothing is ever added to the ring, the plain step writes the output
             e = launch_pconv (g.plan->logM, g.plan->logW, a, st);
         else
-            e = launch_pconv_acc (g.plan->logM, g.plan->logW, PCONV_EMIT, false, a, PConvAcc { d->acc + pos, ring, nullptr, 0 }, st);
+            e = launch_pconv_acc (g.plan->logM, g.plan->logW, PCONV_EMIT, false, false, a, PConvAcc { d->bank[d->cur].acc + pos, ring, nullptr, 0 }, st);
+        if (banks == 2 && e == cudaSuccess)
+        {
+            // the new IR's output mixed over it: weight (n - fade_t0 B + 1) / (fade B) at output sample n (the uniform
+            // schedule's ring stays zero, so the same mode serves it)
+            const ConvBank& nb = d->bank[d->cur ^ 1];
+            const double span = (double) d->fade * B;
+            a.ir = nb.ir[0];
+            const PConvAcc x { nb.acc + pos, ring, nullptr, 0, (float) ((double) ((t - d->fade_t0) * B + 1) / span), (float) (1.0 / span) };
+            e = launch_pconv_acc (g.plan->logM, g.plan->logW, PCONV_EMIT_MIX, false, true, a, x, st);
+        }
     }
     note_kernel ("cfb::pconv_acc_kernel: streaming convolver, %d segments", d->nseg);
     if (e != cudaSuccess)
         return fail_cuda (e, "convolver launch");
     d->t = t + 1;
+    if (banks == 2 && d->t == d->fade_t0 + d->fade) // the crossfade is complete: the new IR's bank becomes the current one
+    {
+        d->cur ^= 1;
+        d->fade = 0;
+    }
+    return 0;
+}
+
+CFB_API int fft_convolver_set_ir (void* ctx, const float* ir, long long ir_length, long long ir_channel_stride, int fade_blocks, void* stream)
+{
+    CFB_TRACE ("fft_convolver_set_ir");
+    ConvCtx* d = as_conv (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    if (d->fade > 0)
+        return fail (FFT_B200_EINVAL, "fft_convolver_set_ir: a crossfade is still running (%lld of %d calls left)", d->fade_t0 + d->fade - d->t, d->fade);
+    if (ir == nullptr || ir_length < 1 || ir_length > d->L || (d->shared_ir ? ir_channel_stride != 0 : ir_channel_stride < ir_length) || fade_blocks < 0
+        || (long long) fade_blocks * d->B > (1LL << 24))
+        return fail (FFT_B200_EINVAL, "fft_convolver_set_ir: bad arguments (1 <= ir_length <= %lld, ir_channel_stride %s, fade_blocks >= 0 and fade_blocks * %d <= 2^24)",
+                     d->L, d->shared_ir ? "0 (shared IR)" : ">= ir_length (per-channel IRs)", d->B);
+    if (misaligned (ir, 4))
+        return fail (FFT_B200_EINVAL, "fft_convolver_set_ir: the IR must be 4-byte aligned");
+    if (classify (ir).kind != Mem::Device)
+        return fail (FFT_B200_EINVAL, "fft_convolver_set_ir needs a device pointer for the IR");
+    int dev = 0;
+    CFB_CUDA (cudaGetDevice (&dev));
+    if (dev != d->device)
+        return fail (FFT_B200_EINVAL, "fft_convolver_set_ir: the context lives on device %d, the current device is %d", d->device, dev);
+    cudaStream_t st = static_cast<cudaStream_t> (stream);
+    ConvBank& nb = d->bank[d->cur ^ 1];
+    if (nb.acc == nullptr) // first call: the second bank and the gather scratch (cudaMalloc may synchronise)
+    {
+        int rc = conv_bank_alloc (d, nb);
+        if (rc == 0 && cudaMalloc (&d->scratch, sizeof (float) * d->scratch_floats) != cudaSuccess)
+            rc = fail (FFT_B200_ECUDA, "fft_convolver_set_ir: out of device memory");
+        if (rc != 0)
+        {
+            conv_bank_free (nb);
+            (void) cudaFree (d->scratch);
+            d->scratch = nullptr;
+            return rc;
+        }
+    }
+    int rc = conv_prepare_ir (d, nb, ir, ir_length, ir_channel_stride, d->scratch, st);
+    if (rc != 0)
+        return rc;
+    const size_t C = (size_t) d->channels;
+    const long long t0 = d->t, B = d->B, ring = d->ring;
+    CFB_CUDA (cudaMemsetAsync (nb.acc, 0, sizeof (float) * C * (size_t) ring, st));
+    // Re-prime: the ring and S of a context that had run with the new IR since call 0.  Only each segment's most recent firing
+    // (t_f = floor(t0 / D) D - 1) adds to samples >= t0 B; re-run it in descending k, the order in which a fresh context made
+    // those additions.  X_q comes from the delay line: the window of the largest segment's firing may already be overwritten in
+    // the input ring.
+    cudaError_t e = cudaSuccess;
+    for (int k = d->nseg - 1; k >= 1 && e == cudaSuccess; --k)
+    {
+        const ConvSegment& g = d->seg[k];
+        const long long D = g.Bk / B, m = t0 / D; // m - 1: the most recent firing, m: the current period
+        const bool sliced = k == d->nseg - 1 && g.P > 1;
+        if (m >= 1)
+        {
+            if (sliced)
+                e = conv_slice (d, nb, k, m - 1, 0, g.Bk / 4, st);
+            if (e == cudaSuccess)
+                e = conv_fire (d, nb, k, m - 1, (m * g.Bk) % ring, true, st);
+        }
+        if (sliced && e == cudaSuccess) // S of the current period in full; the remaining slices of the period rewrite the same values
+            e = conv_slice (d, nb, k, m, 0, g.Bk / 4, st);
+    }
+    if (e != cudaSuccess)
+        return fail_cuda (e, "fft_convolver_set_ir: re-prime launch");
+    if (d->nseg > 1)
+    {
+        // the re-run firings also added into [t0 B - Bmax, t0 B), already emitted; a fresh context holds zeros there
+        const long long from = (t0 * B + d->Bmax) % ring, n1 = from + d->Bmax <= ring ? d->Bmax : ring - from;
+        CFB_CUDA (cudaMemset2DAsync (nb.acc + from, sizeof (float) * ring, 0, sizeof (float) * n1, C, st));
+        if (n1 < d->Bmax)
+            CFB_CUDA (cudaMemset2DAsync (nb.acc, sizeof (float) * ring, 0, sizeof (float) * (d->Bmax - n1), C, st));
+    }
+    if (fade_blocks == 0)
+        d->cur ^= 1;
+    else
+    {
+        d->fade = fade_blocks;
+        d->fade_t0 = t0;
+    }
     return 0;
 }
 
@@ -2351,6 +2510,11 @@ CFB_API int fft_convolver_reset (void* ctx, void* stream)
     ConvCtx* d = as_conv (ctx);
     if (d == nullptr)
         return FFT_B200_EINVAL;
+    if (d->fade > 0) // a running crossfade ends at the new IR
+    {
+        d->cur ^= 1;
+        d->fade = 0;
+    }
     return conv_zero (d, static_cast<cudaStream_t> (stream));
 }
 

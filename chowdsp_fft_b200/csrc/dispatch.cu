@@ -38,12 +38,12 @@ cudaError_t launch_pconv (int logM, int logW, const PConvArgs& args, cudaStream_
         default: return cudaErrorInvalidValue;
     }
 }
-cudaError_t launch_pconv_acc (int logM, int logW, int mode, bool partial, const PConvArgs& args, const PConvAcc& acc, cudaStream_t stream)
+cudaError_t launch_pconv_acc (int logM, int logW, int mode, bool partial, bool from_fdl, const PConvArgs& args, const PConvAcc& acc, cudaStream_t stream)
 {
     switch (logM)
     {
 #define X(n) \
-    case n: return launch_pconv_acc_##n (logW, mode, partial, args, acc, stream);
+    case n: return launch_pconv_acc_##n (logW, mode, partial, from_fdl, args, acc, stream);
         CFB_FOR_SIZES (X)
 #undef X
         default: return cudaErrorInvalidValue;

@@ -65,8 +65,9 @@ void fill_stage_twiddles_rt (int logM, int radix, float2* tw);
 
 // fused partitioned-convolution block step for a REAL plan of 2^(logM+1) samples (one CTA per channel)
 cudaError_t launch_pconv (int logM, int logW, const PConvArgs& args, cudaStream_t stream);
-// its accumulating modes (streaming convolver): mode PCONV_ADD (with or without a partial spectrum) or PCONV_EMIT
-cudaError_t launch_pconv_acc (int logM, int logW, int mode, bool partial, const PConvArgs& args, const PConvAcc& acc, cudaStream_t stream);
+// its accumulating modes (streaming convolver): mode PCONV_ADD (with or without a partial spectrum) or PCONV_EMIT; with from_fdl
+// (X_t read from the delay line) PCONV_ADD (with or without a partial spectrum) or PCONV_EMIT_MIX
+cudaError_t launch_pconv_acc (int logM, int logW, int mode, bool partial, bool from_fdl, const PConvArgs& args, const PConvAcc& acc, cudaStream_t stream);
 // the convolver's sliced tail multiply-accumulate, input-history write and IR partition gather (pconv_kernel.cuh)
 cudaError_t launch_pconv_slice (const PConvSliceArgs& args, cudaStream_t stream);
 cudaError_t launch_conv_input (const ConvInputArgs& args, cudaStream_t stream);
@@ -105,7 +106,7 @@ int& fft_small_mode();
     cudaError_t launch_fft_##n (int kind, int logW, int radix, const FftArgs& args, cudaStream_t stream); \
     cudaError_t launch_fft_juce_##n (int kind, int radix, const FftArgs& args, cudaStream_t stream); \
     cudaError_t launch_pconv_##n (int logW, const PConvArgs& args, cudaStream_t stream);           \
-    cudaError_t launch_pconv_acc_##n (int logW, int mode, bool partial, const PConvArgs& args, const PConvAcc& acc, cudaStream_t stream); \
+    cudaError_t launch_pconv_acc_##n (int logW, int mode, bool partial, bool from_fdl, const PConvArgs& args, const PConvAcc& acc, cudaStream_t stream); \
     cudaError_t launch_stft_##n (int logW, int radix, FftArgs args, cudaStream_t stream);          \
     cudaError_t launch_stft_pipe_##n (int logW, int radix, const FftArgs& args, cudaStream_t stream); \
     cudaError_t launch_istft_##n (int logW, int radix, const FftArgs& args, cudaStream_t stream);  \

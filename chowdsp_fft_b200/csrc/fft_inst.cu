@@ -198,11 +198,11 @@ cudaError_t CFB_CAT (launch_pconv_, CFB_LOGM) (int logW, const PConvArgs& a, cud
 
 namespace
 {
-template <int LOGW, int MODE, bool PARTIAL>
+template <int LOGW, int MODE, bool PARTIAL, bool FROM_FDL = false>
 cudaError_t launch_pconv_acc_one (const PConvArgs& a, const PConvAcc& x, cudaStream_t stream)
 {
     using PL = PConvLaunch<CFB_LOGM>;
-    auto kernel = pconv_acc_kernel<CFB_LOGM, LOGW, MODE, PARTIAL>;
+    auto kernel = pconv_acc_kernel<CFB_LOGM, LOGW, MODE, PARTIAL, FROM_FDL>;
     constexpr int smem_bytes = PL::SMEM_BYTES;
     if (smem_bytes > 48 * 1024)
     {
@@ -216,9 +216,18 @@ cudaError_t launch_pconv_acc_one (const PConvArgs& a, const PConvAcc& x, cudaStr
     count_launch();
     return cudaGetLastError();
 }
+// instances in use: the fused modes, and with FROM_FDL the ones of a second IR bank (ADD, ADD + PARTIAL, EMIT_MIX)
 template <int LOGW>
-cudaError_t launch_pconv_acc_w (int mode, bool partial, const PConvArgs& a, const PConvAcc& x, cudaStream_t stream)
+cudaError_t launch_pconv_acc_w (int mode, bool partial, bool from_fdl, const PConvArgs& a, const PConvAcc& x, cudaStream_t stream)
 {
+    if (from_fdl)
+    {
+        if (mode == PCONV_EMIT_MIX && ! partial)
+            return launch_pconv_acc_one<LOGW, PCONV_EMIT_MIX, false, true> (a, x, stream);
+        if (mode == PCONV_ADD)
+            return partial ? launch_pconv_acc_one<LOGW, PCONV_ADD, true, true> (a, x, stream) : launch_pconv_acc_one<LOGW, PCONV_ADD, false, true> (a, x, stream);
+        return cudaErrorInvalidValue;
+    }
     if (mode == PCONV_EMIT && ! partial)
         return launch_pconv_acc_one<LOGW, PCONV_EMIT, false> (a, x, stream);
     if (mode == PCONV_ADD)
@@ -227,13 +236,13 @@ cudaError_t launch_pconv_acc_w (int mode, bool partial, const PConvArgs& a, cons
 }
 } // namespace
 
-cudaError_t CFB_CAT (launch_pconv_acc_, CFB_LOGM) (int logW, int mode, bool partial, const PConvArgs& a, const PConvAcc& x, cudaStream_t stream)
+cudaError_t CFB_CAT (launch_pconv_acc_, CFB_LOGM) (int logW, int mode, bool partial, bool from_fdl, const PConvArgs& a, const PConvAcc& x, cudaStream_t stream)
 {
     if (logW == 2)
-        return launch_pconv_acc_w<2> (mode, partial, a, x, stream);
+        return launch_pconv_acc_w<2> (mode, partial, from_fdl, a, x, stream);
 #if CFB_LOGM >= 6
     if (logW == 3)
-        return launch_pconv_acc_w<3> (mode, partial, a, x, stream);
+        return launch_pconv_acc_w<3> (mode, partial, from_fdl, a, x, stream);
 #endif
     return cudaErrorInvalidValue;
 }

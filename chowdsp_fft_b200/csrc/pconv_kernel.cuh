@@ -59,24 +59,31 @@ struct PConvLaunch
 // convolver (fft_convolver_*) sums segments of different block sizes in a per-channel accumulator ring:
 //   PCONV_ADD   out[n] += y[n]                       (a segment's delayed contribution, strictly in the future of the ring)
 //   PCONV_EMIT  out[n]  = y[n] + acc[n], acc[n] = 0  (the block being emitted; frees that ring region for later additions)
+//   PCONV_EMIT_MIX  out[n] = (1 - g) out[n] + g (y[n] + acc[n]), acc[n] = 0, g = min(mix_start + n mix_step, 1)  (IR crossfade:
+//                   the new IR's bank mixed over the output the current bank has just emitted)
 // PARTIAL: the accumulator starts from a precomputed partial spectrum S (sum of the older partitions, pconv_slice_kernel) and
 // only the newest spectrum X_t (p = 0) is multiplied in here; slot t % P of the delay line is still written.
+// FROM_FDL: no forward transform; X_t is read from delay-line slot t % P, which an earlier launch has written, and the slot is
+// not written.  The products are those of the fused path, which multiplies the same values from registers, so the result is
+// bitwise the same.  A second IR bank (fft_convolver_set_ir) runs this way on the spectra the current bank has just stored.
 enum PConvMode
 {
     PCONV_WRITE = 0,
     PCONV_ADD = 1,
-    PCONV_EMIT = 2
+    PCONV_EMIT = 2,
+    PCONV_EMIT_MIX = 3
 };
 
 struct PConvAcc
 {
-    float* acc;         // PCONV_EMIT: channel c's ring region at acc + c * acc_stride (N/2 samples)
+    float* acc;         // PCONV_EMIT / PCONV_EMIT_MIX: channel c's ring region at acc + c * acc_stride (N/2 samples)
     long long acc_stride;
     const float* S;     // PARTIAL: channel c's partial spectrum at S + c * s_stride (N floats, unordered, unscaled)
     long long s_stride;
+    float mix_start, mix_step; // PCONV_EMIT_MIX: weight of the new result at output sample 0 and its step per sample
 };
 
-template <int LOGM, int LOGW, int MODE = PCONV_WRITE, bool PARTIAL = false>
+template <int LOGM, int LOGW, int MODE = PCONV_WRITE, bool PARTIAL = false, bool FROM_FDL = false>
 FFT_HD void pconv_body (const PConvArgs& a, const PConvAcc& x = PConvAcc {})
 {
     constexpr int R = 16;
@@ -95,7 +102,8 @@ FFT_HD void pconv_body (const PConvArgs& a, const PConvAcc& x = PConvAcc {})
     const int c = active ? (int) c0 : a.channels - 1;
 
     // 1. forward transform of the window; the unordered spectrum stays in shared memory (staging image)
-    fft_core<LOGM, R, R2C, LOGW, false, true, false> (a.in + (long long) c * a.in_stride, nullptr, true, j, smem, a.tw, a.rtw);
+    if constexpr (! FROM_FDL)
+        fft_core<LOGM, R, R2C, LOGW, false, true, false> (a.in + (long long) c * a.in_stride, nullptr, true, j, smem, a.tw, a.rtw);
 
     // 2. this thread's slice of the spectrum: PAIRS x (4 re lanes, 4 im lanes); float offset of the re quad
     int off[PAIRS];
@@ -106,12 +114,20 @@ FFT_HD void pconv_body (const PConvArgs& a, const PConvAcc& x = PConvAcc {})
     {
         const int pr = j + i * T;
         off[i] = (pr / (W / 4)) * 2 * W + (pr % (W / 4)) * 4;
-        xr[i] = lds4 (sf + upad (off[i], LOGW));
-        xi[i] = lds4 (sf + upad (off[i] + W, LOGW));
-        if (active)
+        if constexpr (FROM_FDL)
         {
-            *reinterpret_cast<float4*> (slot + off[i]) = xr[i];     // delay-line write (linear across the channel's threads)
-            *reinterpret_cast<float4*> (slot + off[i] + W) = xi[i];
+            xr[i] = ld_stream4 (slot + off[i]);
+            xi[i] = ld_stream4 (slot + off[i] + W);
+        }
+        else
+        {
+            xr[i] = lds4 (sf + upad (off[i], LOGW));
+            xi[i] = lds4 (sf + upad (off[i] + W, LOGW));
+            if (active)
+            {
+                *reinterpret_cast<float4*> (slot + off[i]) = xr[i];     // delay-line write (linear across the channel's threads)
+                *reinterpret_cast<float4*> (slot + off[i] + W) = xi[i];
+            }
         }
         if constexpr (PARTIAL)
         {
@@ -188,15 +204,23 @@ FFT_HD void pconv_body (const PConvArgs& a, const PConvAcc& x = PConvAcc {})
         if (active)
         {
             float2* o2 = reinterpret_cast<float2*> (outc) + j;
-            float2* acc2 = MODE == PCONV_EMIT ? reinterpret_cast<float2*> (x.acc + (long long) c * x.acc_stride - M) + j : nullptr;
+            float2* acc2 = MODE != PCONV_ADD ? reinterpret_cast<float2*> (x.acc + (long long) c * x.acc_stride - M) + j : nullptr;
 #pragma unroll
             for (int m = R / 2; m < R; ++m)
             {
                 if constexpr (MODE == PCONV_ADD)
                     o2[m * T] = f2_add (o2[m * T], v[m]);
-                else
+                else if constexpr (MODE == PCONV_EMIT)
                 {
                     o2[m * T] = f2_add (v[m], acc2[m * T]);
+                    acc2[m * T] = make_float2 (0.f, 0.f);
+                }
+                else
+                {
+                    const float2 r = f2_add (v[m], acc2[m * T]), o = o2[m * T];
+                    const float n = (float) (2 * (j + m * T) - M); // output sample of r.x
+                    const float g0 = fminf (fmaf (n, x.mix_step, x.mix_start), 1.f), g1 = fminf (fmaf (n + 1.f, x.mix_step, x.mix_start), 1.f);
+                    o2[m * T] = make_float2 (fmaf (g0, r.x, (1.f - g0) * o.x), fmaf (g1, r.y, (1.f - g1) * o.y));
                     acc2[m * T] = make_float2 (0.f, 0.f);
                 }
             }
@@ -210,11 +234,11 @@ __global__ void __launch_bounds__ (PConvLaunch<LOGM>::THREADS, (PConvLaunch<LOGM
     pconv_body<LOGM, LOGW> (a);
 }
 
-// the accumulating modes (streaming convolver): one instance per (MODE, PARTIAL) in use
-template <int LOGM, int LOGW, int MODE, bool PARTIAL>
+// the accumulating modes (streaming convolver): one instance per (MODE, PARTIAL, FROM_FDL) in use
+template <int LOGM, int LOGW, int MODE, bool PARTIAL, bool FROM_FDL = false>
 __global__ void __launch_bounds__ (PConvLaunch<LOGM>::THREADS, (PConvLaunch<LOGM>::THREADS <= 256 ? 2 : 1)) pconv_acc_kernel (const PConvArgs a, const PConvAcc x)
 {
-    pconv_body<LOGM, LOGW, MODE, PARTIAL> (a, x);
+    pconv_body<LOGM, LOGW, MODE, PARTIAL, FROM_FDL> (a, x);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -108,13 +108,29 @@ int fft_partitioned_convolve_step (void* setup, const float* windows, long long 
      fft_convolver_create    allocates and zeroes the state and transforms the IR partitions (synchronous on `stream`);
                              16 <= block_size <= 16384, a power of two; ir_length >= 1; ir_channel_stride 0 or >= ir_length
      fft_convolver_process   one block per channel; input / output 8-byte aligned with even strides; stream-ordered
-     fft_convolver_reset     back to silence (the IR is kept); stream-ordered
+     fft_convolver_set_ir    replaces the IR on a live context, instantly or with a crossfade (below); stream-ordered
+     fft_convolver_reset     back to silence (the newest IR is kept, a running crossfade ends); stream-ordered
      fft_convolver_segments  up to max_segments (block size, partitions) pairs (either array may be NULL); returns the count
-     fft_convolver_destroy   waits for the device, then frees the context
+     fft_convolver_destroy   waits for the device, then frees the context (both IR banks)
    Device pointers only.  Calls on one context must be ordered on one stream, on the device that was current at create,
-   and a context must not be used from two threads at the same time. */
+   and a context must not be used from two threads at the same time.
+
+   fft_convolver_set_ir (ctx, ir, ir_length, ir_channel_stride, fade_blocks, stream): switches to the IR h' at ir (layout as
+   at create) while audio runs, without cutting the reverb tail of what was already played.  With t0 the number of process
+   calls since create / reset, call t >= t0 writes
+       y[n] = (1 - g[n]) (h * x)[n] + g[n] (h' * x)[n],   g[n] = min((n - t0 B + 1) / (fade_blocks B), 1),
+   both convolutions over the whole input history; fade_blocks = 0 switches at once (g = 1 from call t0 on).  Once the fade
+   is over, every output is bit-identical to that of a context created with h' (zero-padded to the create-time length) and
+   fed the same input from its first call.  1 <= ir_length <= the ir_length given at create (the schedule is fixed; a
+   shorter IR is zero-padded); ir_channel_stride 0 for a context created with a shared IR, else >= ir_length; 4-byte aligned
+   device pointer; fade_blocks >= 0 with fade_blocks * B <= 2^24.  During a fade every process call runs both IRs (about
+   twice the work); a call while a fade is running, or with a bad argument, returns FFT_B200_EINVAL and leaves the context
+   unchanged.  Stream-ordered: ir is read when `stream` reaches the call.  The first call on a context allocates the second
+   IR bank and a gather buffer and may synchronise, like create; to keep that off an audio thread, call it once at start-up
+   with the current IR (fade_blocks = 0).  Every later call allocates nothing and does not block the host. */
 int fft_convolver_create (int channels, int block_size, const float* ir, long long ir_length, long long ir_channel_stride, void* stream, void** ctx_out);
 int fft_convolver_process (void* ctx, const float* input, long long input_stride, float* output, long long output_stride, void* stream);
+int fft_convolver_set_ir (void* ctx, const float* ir, long long ir_length, long long ir_channel_stride, int fade_blocks, void* stream);
 int fft_convolver_reset (void* ctx, void* stream);
 int fft_convolver_segments (void* ctx, int* block_sizes, int* partitions, int max_segments);
 int fft_convolver_destroy (void* ctx);
