@@ -68,6 +68,11 @@ def lib() -> C.CDLL:
         "fft_convolver_reset": (i, [vp, vp]),
         "fft_convolver_segments": (i, [vp, C.POINTER(C.c_int), C.POINTER(C.c_int), i]),
         "fft_convolver_destroy": (i, [vp]),
+        "fft_stft_stream_create": (i, [vp, i, ll, i, vp, vp, f, i, vp, C.POINTER(vp)]),
+        "fft_stft_stream_analyze": (i, [vp, vp, ll, i, vp, ll, ll, vp]),
+        "fft_stft_stream_synthesize": (i, [vp, vp, ll, ll, i, vp, ll, vp]),
+        "fft_stft_stream_reset": (i, [vp, vp]),
+        "fft_stft_stream_destroy": (i, [vp]),
         "fft_dist_phase": (i, [vp, i, i, i, vp, vp, i, vp]),
         "fft_dist_phase0_peer": (i, [vp, i, i, vp, C.POINTER(vp), i, vp]),
         "fft_dist_alloc": (vp, [C.c_size_t]),
@@ -104,6 +109,6 @@ EXPORTED = (
     "fft_bytes_required", "fft_new_setup", "fft_new_setup_preallocated", "fft_destroy_setup",
     "fft_simd_width_bytes", "fft_transform", "fft_transform_unordered", "fft_convolve_unordered",
     "fft_accumulate", "aligned_malloc", "aligned_free", "fft_transform_batched", "fft_transform_strided", "fft_stft_forward", "fft_istft_overlap_add", "fft_juce_perform_batched", "fft_juce_real_forward_batched", "fft_juce_real_inverse_batched",
-    "fft_convolve_unordered_batched", "fft_accumulate_batched", "fft_partitioned_convolve_step", "fft_convolver_create", "fft_convolver_process", "fft_convolver_set_ir", "fft_convolver_reset", "fft_convolver_segments", "fft_convolver_destroy", "fft_dist_phase", "fft_dist_phase0_peer", "fft_dist_alloc", "fft_dist_free", "fft_dist_ipc_export", "fft_dist_ipc_open", "fft_dist_ipc_close", "fft_dist_create", "fft_dist_blob_bytes", "fft_dist_export", "fft_dist_connect", "fft_dist_transform", "fft_dist_natural_buffer", "fft_dist_status", "fft_dist_phase_ms", "fft_dist_destroy", "fft_large_factors", "fft_b200_set_tuning", "fft_b200_last_error", "fft_b200_last_kernel", "fft_b200_clear_error",
+    "fft_convolve_unordered_batched", "fft_accumulate_batched", "fft_partitioned_convolve_step", "fft_convolver_create", "fft_convolver_process", "fft_convolver_set_ir", "fft_convolver_reset", "fft_convolver_segments", "fft_convolver_destroy", "fft_stft_stream_create", "fft_stft_stream_analyze", "fft_stft_stream_synthesize", "fft_stft_stream_reset", "fft_stft_stream_destroy", "fft_dist_phase", "fft_dist_phase0_peer", "fft_dist_alloc", "fft_dist_free", "fft_dist_ipc_export", "fft_dist_ipc_open", "fft_dist_ipc_close", "fft_dist_create", "fft_dist_blob_bytes", "fft_dist_export", "fft_dist_connect", "fft_dist_transform", "fft_dist_natural_buffer", "fft_dist_status", "fft_dist_phase_ms", "fft_dist_destroy", "fft_large_factors", "fft_b200_set_tuning", "fft_b200_last_error", "fft_b200_last_kernel", "fft_b200_clear_error",
     "fft_b200_launch_count", "fft_b200_device_available",
 )

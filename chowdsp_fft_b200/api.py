@@ -235,6 +235,39 @@ def fft_convolver_destroy(ctx: int) -> None:
     _check(lib().fft_convolver_destroy(ctx))
 
 
+# ---- streaming STFT (chowdsp_fft_b200.h: fft_stft_stream_create ... fft_stft_stream_destroy) ----
+def fft_stft_stream_create(setup: int, channels: int, hop: int, max_frames: int, analysis_window=None, synthesis_window=None,
+                           scale: float = 1.0, ordered: bool = True, stream=None) -> int:
+    """Context for block-by-block STFT analysis and overlap-add synthesis of `channels` signals: hop = N/2, N/4 or N/8 of the
+    REAL plan `setup` (N = 128 .. 8192), up to max_frames frames per call; the windows (None = rectangular) are copied."""
+    ctx = C.c_void_p()
+    _check(lib().fft_stft_stream_create(setup, channels, hop, max_frames, _addr(analysis_window), _addr(synthesis_window), scale,
+                                        int(ordered), _stream(stream), C.byref(ctx)))
+    return ctx.value
+
+
+def fft_stft_stream_analyze(ctx: int, input, input_stride: int, frames: int, spectra, spec_channel_stride: int,
+                            spec_frame_stride: int, stream=None) -> None:
+    """frames * hop new samples per channel in, `frames` spectra per channel out."""
+    _check(lib().fft_stft_stream_analyze(ctx, _addr(input), input_stride, frames, _addr(spectra), spec_channel_stride,
+                                         spec_frame_stride, _stream(stream)))
+
+
+def fft_stft_stream_synthesize(ctx: int, spectra, spec_channel_stride: int, spec_frame_stride: int, frames: int, output,
+                               output_stride: int, stream=None) -> None:
+    """`frames` spectra per channel in, frames * hop finished overlap-add samples per channel out."""
+    _check(lib().fft_stft_stream_synthesize(ctx, _addr(spectra), spec_channel_stride, spec_frame_stride, frames, _addr(output),
+                                            output_stride, _stream(stream)))
+
+
+def fft_stft_stream_reset(ctx: int, stream=None) -> None:
+    _check(lib().fft_stft_stream_reset(ctx, _stream(stream)))
+
+
+def fft_stft_stream_destroy(ctx: int) -> None:
+    _check(lib().fft_stft_stream_destroy(ctx))
+
+
 def set_tuning(key: str, value: int) -> None:
     """Benchmark/sweep hook (fft_b200_set_tuning)."""
     _check(lib().fft_b200_set_tuning(key.encode(), int(value)))

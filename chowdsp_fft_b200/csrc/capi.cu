@@ -2544,6 +2544,245 @@ CFB_API int fft_convolver_destroy (void* ctx)
     return 0;
 }
 
+// ---- streaming STFT: analysis and overlap-add synthesis contexts (chowdsp_fft_b200.h: fft_stft_stream_*) ----------------
+namespace
+{
+constexpr uint64_t kStftStreamMagic = 0x4346425354465331ull; // "CFBSTFS1"
+
+struct StftStreamCtx
+{
+    uint64_t magic;
+    int channels = 0, max_frames = 0, device = 0;
+    bool ordered = false;
+    long long N = 0, hop = 0;
+    float scale = 1.f;
+    Plan* plan = nullptr;           // the context's own REAL plan of N points (same unordered layout as the caller's)
+    Tables tables;                  // its radix-16 tables (ristft_carry_kernel)
+    float* awin = nullptr;          // copies of the windows (N floats each), nullptr = rectangular
+    float* swin = nullptr;
+    // analysis: mirrored input ring per channel, [ring | ring | max_frames hop] floats at hist + c * hist_stride.  Padded-signal
+    // sample q (N - hop zeros, then the input) is stored at q % ring and q % ring + ring, by one conv_input_kernel launch per call
+    float* hist = nullptr;
+    long long ring = 0, hist_stride = 0;
+    long long a_frames = 0;         // spectra produced since create / reset
+    // synthesis: the N - hop carried overlap-add sums per channel (ristft_carry_kernel's accumulators)
+    float* carry = nullptr;
+};
+
+StftStreamCtx* as_stft_stream (void* ctx)
+{
+    auto* d = static_cast<StftStreamCtx*> (ctx);
+    if (d == nullptr || (reinterpret_cast<uintptr_t> (d) & 7) != 0 || d->magic != kStftStreamMagic)
+    {
+        fail (chowdsp::fft::FFT_B200_EINVAL, "invalid streaming STFT context %p", ctx);
+        return nullptr;
+    }
+    return d;
+}
+
+void stft_stream_free (StftStreamCtx* d)
+{
+    (void) cudaFree (d->awin);
+    (void) cudaFree (d->swin);
+    (void) cudaFree (d->hist);
+    (void) cudaFree (d->carry);
+    if (d->plan != nullptr)
+        chowdsp::fft::fft_destroy_setup (d->plan);
+    d->magic = 0;
+    delete d;
+}
+
+int stft_stream_zero (StftStreamCtx* d, cudaStream_t st)
+{
+    const size_t C = (size_t) d->channels;
+    CFB_CUDA (cudaMemsetAsync (d->hist, 0, sizeof (float) * C * (size_t) d->hist_stride, st));
+    CFB_CUDA (cudaMemsetAsync (d->carry, 0, sizeof (float) * C * (size_t) (d->N - d->hop), st));
+    d->a_frames = 0;
+    return 0;
+}
+
+int stft_stream_check_device (const StftStreamCtx* d, const char* fn)
+{
+    int dev = 0;
+    CFB_CUDA (cudaGetDevice (&dev));
+    if (dev != d->device)
+        return fail (chowdsp::fft::FFT_B200_EINVAL, "%s: the context lives on device %d, the current device is %d", fn, d->device, dev);
+    return 0;
+}
+} // namespace
+
+CFB_API int fft_stft_stream_create (void* setup, int channels, long long hop, int max_frames, const float* analysis_window, const float* synthesis_window, float scale,
+                                    int ordered, void* stream, void** ctx_out)
+{
+    CFB_TRACE ("fft_stft_stream_create");
+    if (ctx_out == nullptr)
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_create: null ctx_out");
+    *ctx_out = nullptr;
+    Plan* p = as_plan (setup);
+    if (p == nullptr)
+        return FFT_B200_EINVAL;
+    if (p->is_complex || p->mixed || p->logM < 6 || p->logM > 12)
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_create needs a REAL power-of-two plan with 128 <= N <= 8192");
+    if (hop * 2 != p->N && hop * 4 != p->N && hop * 8 != p->N)
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_create: hop %lld is not N/2, N/4 or N/8 (N = %d)", hop, p->N);
+    if (channels < 1 || max_frames < 1 || (long long) channels * max_frames > 0x7fffffffLL || (long long) max_frames * hop > (1LL << 28))
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_create: bad arguments (channels >= 1, max_frames >= 1)");
+    for (const float* w : { analysis_window, synthesis_window })
+        if (w != nullptr && misaligned (w, 4))
+            return fail (FFT_B200_EINVAL, "fft_stft_stream_create: the windows must be 4-byte aligned");
+    if (! device_available())
+        return fail (FFT_B200_ENODEVICE, "no usable CUDA device: chowdsp_fft_b200 has no CPU fallback");
+    auto* d = new (std::nothrow) StftStreamCtx();
+    if (d == nullptr)
+        return fail (FFT_B200_ECUDA, "out of host memory");
+    d->magic = kStftStreamMagic;
+    d->channels = channels;
+    d->max_frames = max_frames;
+    d->ordered = ordered != 0;
+    d->N = p->N;
+    d->hop = hop;
+    d->scale = scale;
+    // ring >= (N - hop) + 2 max_frames hop: a call's frames span (N - hop) + frames hop samples, and a call whose span crosses
+    // the ring's end reads the low copy, whose entries for that span no earlier call can have wrapped over (see analyze).
+    // A multiple of 4 floats: every frame start keeps the 16-byte alignment of an offline frame at f hop.
+    const long long span_max = (long long) max_frames * hop;
+    d->ring = (p->N - hop + 2 * span_max + 3) & ~3LL;
+    d->hist_stride = 2 * d->ring + span_max;
+    cudaStream_t st = static_cast<cudaStream_t> (stream);
+    const size_t C = (size_t) channels, wbytes = sizeof (float) * (size_t) p->N;
+    int rc = 0;
+    cudaError_t e = cudaGetDevice (&d->device);
+    if (e == cudaSuccess)
+    {
+        d->plan = static_cast<Plan*> (chowdsp::fft::fft_new_setup (p->N, chowdsp::fft::FFT_REAL, p->logW == 3));
+        if (d->plan == nullptr || d->plan->logW != p->logW)
+            rc = fail (FFT_B200_ECUDA, "fft_stft_stream_create: could not create the context's plan");
+    }
+    if (e == cudaSuccess && rc == 0)
+        rc = plan_tables (d->plan, d->tables, 16);
+    if (e == cudaSuccess && rc == 0 && analysis_window != nullptr && (e = cudaMalloc (&d->awin, wbytes)) == cudaSuccess)
+        e = cudaMemcpyAsync (d->awin, analysis_window, wbytes, cudaMemcpyDefault, st);
+    if (e == cudaSuccess && rc == 0 && synthesis_window != nullptr && (e = cudaMalloc (&d->swin, wbytes)) == cudaSuccess)
+        e = cudaMemcpyAsync (d->swin, synthesis_window, wbytes, cudaMemcpyDefault, st);
+    if (e == cudaSuccess && rc == 0 && (e = cudaMalloc (&d->hist, sizeof (float) * C * (size_t) d->hist_stride)) == cudaSuccess)
+        e = cudaMalloc (&d->carry, sizeof (float) * C * (size_t) (p->N - hop));
+    if (e == cudaSuccess && rc == 0)
+        rc = stft_stream_zero (d, st);
+    if (e == cudaSuccess && rc == 0)
+        e = cudaStreamSynchronize (st); // the windows may be freed by the caller once create returns
+    if (e != cudaSuccess && rc == 0)
+        rc = fail_cuda (e, "fft_stft_stream_create");
+    if (rc != 0)
+    {
+        (void) cudaStreamSynchronize (st);
+        stft_stream_free (d);
+        return rc;
+    }
+    *ctx_out = d;
+    return 0;
+}
+
+CFB_API int fft_stft_stream_analyze (void* ctx, const float* input, long long input_stride, int frames, float* spectra, long long spec_channel_stride, long long spec_frame_stride,
+                                     void* stream)
+{
+    CFB_TRACE ("fft_stft_stream_analyze");
+    StftStreamCtx* d = as_stft_stream (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    const int C = d->channels;
+    if (input == nullptr || spectra == nullptr || frames < 1 || frames > d->max_frames)
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_analyze: bad arguments (non-null buffers, 1 <= frames <= max_frames = %d)", d->max_frames);
+    if (misaligned (input, 8, input_stride, C))
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_analyze: the input must be 8-byte aligned with an even channel stride");
+    if (misaligned (spectra, d->ordered ? 8 : 16, spec_frame_stride, frames, spec_channel_stride, C))
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_analyze: every spectrum must start on an 8-byte boundary (16-byte for unordered spectra): check the base pointer and strides");
+    if (classify (input).kind != Mem::Device || classify (spectra).kind != Mem::Device)
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_analyze needs device pointers");
+    int rc = stft_stream_check_device (d, "fft_stft_stream_analyze");
+    if (rc != 0)
+        return rc;
+    cudaStream_t st = static_cast<cudaStream_t> (stream);
+    // this call's frames cover padded samples [P0, P0 + span), the new ones are the last frames hop of them
+    const long long hop = d->hop, ring = d->ring, n_new = (long long) frames * hop, span = d->N - hop + n_new;
+    const long long P0 = d->a_frames * hop, b = P0 % ring, w = (P0 + d->N - hop) % ring;
+    // The high copy [ring, 2 ring) always holds the newest sample of every residue (a write that crosses the ring's end lands
+    // its wrapped part there through the low copy's overflow).  A span that crosses the end reads the low copy instead:
+    // then b > ring - span >= ring - (N - hop) - max_frames hop >= max_frames hop, so a write that wrapped at P0 - b ended
+    // before P0, and every sample of [P0, P0 + ring - b) sits at its own place in the low copy.
+    const long long base = b + span <= ring ? ring + b : b;
+    const cudaError_t e = launch_conv_input (ConvInputArgs { input, input_stride, d->hist, d->hist_stride, C, (int) (n_new / 2), w, ring }, st);
+    if (e != cudaSuccess)
+        return fail_cuda (e, "streaming STFT input launch");
+    rc = enqueue_transform (d->plan, d->hist + base, spectra, C, frames, d->hist_stride, hop, spec_channel_stride, spec_frame_stride, FFT_FORWARD, d->ordered, st, d->awin);
+    if (rc != 0)
+        return rc;
+    d->a_frames += frames;
+    return 0;
+}
+
+CFB_API int fft_stft_stream_synthesize (void* ctx, const float* spectra, long long spec_channel_stride, long long spec_frame_stride, int frames, float* output, long long output_stride,
+                                        void* stream)
+{
+    CFB_TRACE ("fft_stft_stream_synthesize");
+    StftStreamCtx* d = as_stft_stream (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    const int C = d->channels;
+    if (spectra == nullptr || output == nullptr || frames < 1 || frames > d->max_frames)
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_synthesize: bad arguments (non-null buffers, 1 <= frames <= max_frames = %d)", d->max_frames);
+    if (misaligned (spectra, d->ordered ? 8 : 16, spec_frame_stride, frames, spec_channel_stride, C))
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_synthesize: every spectrum must start on an 8-byte boundary (16-byte for unordered spectra): check the base pointer and strides");
+    if (misaligned (output, 8, output_stride, C))
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_synthesize: the output must be 8-byte aligned with an even channel stride");
+    if (classify (spectra).kind != Mem::Device || classify (output).kind != Mem::Device)
+        return fail (FFT_B200_EINVAL, "fft_stft_stream_synthesize needs device pointers");
+    const int rc = stft_stream_check_device (d, "fft_stft_stream_synthesize");
+    if (rc != 0)
+        return rc;
+    FftArgs a {};
+    a.in = spectra;
+    a.out = output;
+    a.in_inner = spec_frame_stride;
+    a.in_outer = spec_channel_stride;
+    a.out_inner = d->hop;
+    a.out_outer = output_stride;
+    a.inner = frames;
+    a.batch = C * frames;
+    a.tw = d->tables.tw;
+    a.rtw = d->tables.rtw;
+    a.window = d->swin;
+    a.seg_frames = frames;
+    a.nseg = 1;
+    a.scale = d->scale;
+    const int logW = d->ordered ? 0 : d->plan->logW, hq = (int) (d->hop * 16 / d->N);
+    const cudaError_t e = launch_ristft (d->plan->logM, hq, logW, a, static_cast<cudaStream_t> (stream), reinterpret_cast<float2*> (d->carry));
+    if (e != cudaSuccess)
+        return fail_cuda (e, "streaming overlap-add synthesis launch");
+    note_kernel ("cfb::ristft_carry_kernel<%d,%d,%d>", d->plan->logM, hq, logW);
+    return 0;
+}
+
+CFB_API int fft_stft_stream_reset (void* ctx, void* stream)
+{
+    CFB_TRACE ("fft_stft_stream_reset");
+    StftStreamCtx* d = as_stft_stream (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    const int rc = stft_stream_check_device (d, "fft_stft_stream_reset");
+    return rc != 0 ? rc : stft_stream_zero (d, static_cast<cudaStream_t> (stream));
+}
+
+CFB_API int fft_stft_stream_destroy (void* ctx)
+{
+    StftStreamCtx* d = as_stft_stream (ctx);
+    if (d == nullptr)
+        return FFT_B200_EINVAL;
+    (void) cudaDeviceSynchronize(); // work queued on any stream may still use the buffers
+    stft_stream_free (d);
+    (void) cudaGetLastError();
+    return 0;
+}
+
 CFB_API int fft_large_factors (void* setup, int* l1, int* l2, int* l3)
 {
     Plan* p = as_plan (setup);

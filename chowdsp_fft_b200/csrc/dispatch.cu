@@ -150,12 +150,12 @@ cudaError_t launch_stft_pipe (int logM, int logW, int radix, const FftArgs& args
         default: return cudaErrorInvalidValue;
     }
 }
-cudaError_t launch_ristft (int logM, int hq, int logW, const FftArgs& args, cudaStream_t stream)
+cudaError_t launch_ristft (int logM, int hq, int logW, const FftArgs& args, cudaStream_t stream, float2* carry)
 {
     switch (logM)
     {
 #define X(n) \
-    case n: return launch_ristft_##n (hq, logW, args, stream);
+    case n: return launch_ristft_##n (hq, logW, args, stream, carry);
         CFB_FOR_SIZES (X)
 #undef X
         default: return cudaErrorInvalidConfiguration;

@@ -34,9 +34,10 @@ cudaError_t launch_stft_pipe (int logM, int logW, int radix, const FftArgs& args
 // spectrum frame / channel strides, args.out_inner = hop (0 < hop <= N), args.out_outer = signal channel stride,
 // args.inner = frames per channel, args.seg_frames (multiple of transforms_per_cta) and args.nseg = segmentation
 cudaError_t launch_istft (int logM, int logW, int radix, const FftArgs& args, cudaStream_t stream);
-// overlap-add synthesis with register accumulators (ristft_kernel: complex lengths 2^9 .. 2^12, hq = hop / (2 T) in {2, 4, 8});
-// cudaErrorInvalidConfiguration = no such instance
-cudaError_t launch_ristft (int logM, int hq, int logW, const FftArgs& args, cudaStream_t stream);
+// overlap-add synthesis with register accumulators (ristft_kernel: complex lengths 2^6 .. 2^12, hq = hop / (2 T) in {2, 4, 8});
+// cudaErrorInvalidConfiguration = no such instance.  carry != nullptr: streaming synthesis (ristft_carry_kernel, args.nseg = 1,
+// args.seg_frames = args.inner) whose accumulators start from and end in carry, (N - hop) / 2 float2 per channel
+cudaError_t launch_ristft (int logM, int hq, int logW, const FftArgs& args, cudaStream_t stream, float2* carry = nullptr);
 int transforms_per_cta (int logM, int radix);
 // persistent TMA-pipelined variant (pipe_kernels.cuh) for complex lengths 2^13 / 2^14, logW 0 or 3, plain batches
 // (args.inner == args.batch) whose input rows are 16-byte aligned
@@ -110,7 +111,7 @@ int& fft_small_mode();
     cudaError_t launch_stft_##n (int logW, int radix, FftArgs args, cudaStream_t stream);          \
     cudaError_t launch_stft_pipe_##n (int logW, int radix, const FftArgs& args, cudaStream_t stream); \
     cudaError_t launch_istft_##n (int logW, int radix, const FftArgs& args, cudaStream_t stream);  \
-    cudaError_t launch_ristft_##n (int hq, int logW, const FftArgs& args, cudaStream_t stream);    \
+    cudaError_t launch_ristft_##n (int hq, int logW, const FftArgs& args, cudaStream_t stream, float2* carry); \
     int transforms_per_cta_##n (int radix);                                                    \
     int has_radix32_##n();                                                                     \
     int stage_twiddle_len_##n (int radix);                                                     \

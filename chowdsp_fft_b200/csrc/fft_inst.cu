@@ -383,54 +383,64 @@ cudaError_t launch_istft_r (int logW, const FftArgs& a, cudaStream_t stream)
 }
 } // namespace
 
-// overlap-add synthesis with register accumulators (ristft_kernel): hq = hop / (2 T) in {2, 4, 8}; cudaErrorInvalidConfiguration = no such instance
+// overlap-add synthesis with register accumulators (ristft_kernel): hq = hop / (2 T) in {2, 4, 8}; cudaErrorInvalidConfiguration = no such instance.
+// carry != nullptr: the streaming variant (ristft_carry_kernel), one item per channel, accumulators loaded from and stored to carry
 #if CFB_LOGM >= 6 && CFB_LOGM <= 12
 namespace
 {
-template <int HQ, int LOGW>
-cudaError_t launch_ristft_one (const FftArgs& a, cudaStream_t stream)
+template <int HQ, int LOGW, bool CARRY>
+cudaError_t launch_ristft_one (const FftArgs& a, float2* carry, cudaStream_t stream)
 {
     using L = Launch<CFB_LOGM, 16>;
-    auto kernel = ristft_kernel<CFB_LOGM, HQ, LOGW>;
     constexpr int smem_bytes = LOGW != 0 ? L::SMEM_BYTES_UNORD : L::SMEM_BYTES;
     if (smem_bytes > 48 * 1024)
     {
-        const cudaError_t e = cudaFuncSetAttribute (kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+        const cudaError_t e = CARRY ? cudaFuncSetAttribute (ristft_carry_kernel<CFB_LOGM, HQ, LOGW>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes)
+                                    : cudaFuncSetAttribute (ristft_kernel<CFB_LOGM, HQ, LOGW>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
         if (e != cudaSuccess)
             return e;
     }
     const long long items = (long long) (a.batch / a.inner) * a.nseg;
     if (items <= 0)
         return cudaSuccess;
-    kernel<<<(unsigned) ((items + L::PER_CTA - 1) / L::PER_CTA), L::THREADS, smem_bytes, stream>>> (a);
+    const unsigned grid = (unsigned) ((items + L::PER_CTA - 1) / L::PER_CTA);
+    if constexpr (CARRY)
+        ristft_carry_kernel<CFB_LOGM, HQ, LOGW><<<grid, L::THREADS, smem_bytes, stream>>> (a, carry);
+    else
+        ristft_kernel<CFB_LOGM, HQ, LOGW><<<grid, L::THREADS, smem_bytes, stream>>> (a);
     count_launch();
     return cudaGetLastError();
 }
-template <int HQ>
-cudaError_t launch_ristft_h (int logW, const FftArgs& a, cudaStream_t stream)
+template <int HQ, bool CARRY>
+cudaError_t launch_ristft_h (int logW, const FftArgs& a, float2* carry, cudaStream_t stream)
 {
     switch (logW)
     {
-        case 0: return launch_ristft_one<HQ, 0> (a, stream);
-        case 2: return launch_ristft_one<HQ, 2> (a, stream);
-        case 3: return launch_ristft_one<HQ, 3> (a, stream);
+        case 0: return launch_ristft_one<HQ, 0, CARRY> (a, carry, stream);
+        case 2: return launch_ristft_one<HQ, 2, CARRY> (a, carry, stream);
+        case 3: return launch_ristft_one<HQ, 3, CARRY> (a, carry, stream);
+        default: return cudaErrorInvalidConfiguration;
+    }
+}
+template <bool CARRY>
+cudaError_t launch_ristft_c (int hq, int logW, const FftArgs& a, float2* carry, cudaStream_t stream)
+{
+    switch (hq)
+    {
+        case 2: return launch_ristft_h<2, CARRY> (logW, a, carry, stream);
+        case 4: return launch_ristft_h<4, CARRY> (logW, a, carry, stream);
+        case 8: return launch_ristft_h<8, CARRY> (logW, a, carry, stream);
         default: return cudaErrorInvalidConfiguration;
     }
 }
 } // namespace
 #endif
-cudaError_t CFB_CAT (launch_ristft_, CFB_LOGM) (int hq, int logW, const FftArgs& a, cudaStream_t stream)
+cudaError_t CFB_CAT (launch_ristft_, CFB_LOGM) (int hq, int logW, const FftArgs& a, cudaStream_t stream, float2* carry)
 {
 #if CFB_LOGM >= 6 && CFB_LOGM <= 12
-    switch (hq)
-    {
-        case 2: return launch_ristft_h<2> (logW, a, stream);
-        case 4: return launch_ristft_h<4> (logW, a, stream);
-        case 8: return launch_ristft_h<8> (logW, a, stream);
-        default: return cudaErrorInvalidConfiguration;
-    }
+    return carry != nullptr ? launch_ristft_c<true> (hq, logW, a, carry, stream) : launch_ristft_c<false> (hq, logW, a, nullptr, stream);
 #else
-    (void) hq; (void) logW; (void) a; (void) stream;
+    (void) hq; (void) logW; (void) a; (void) stream; (void) carry;
     return cudaErrorInvalidConfiguration;
 #endif
 }

@@ -1667,9 +1667,13 @@ FFT_HD void istft_body (const FftArgs& a)
 // these sizes, tools/stft_sweep.py).  Segments other than a channel's first recompute a halo of N / hop - 1 frames.
 // a.in_inner / in_outer: floats between frames / channels of the spectra; a.out_inner = hop; a.out_outer: floats between channels
 // of the signal; a.nseg, a.seg_frames: segments per channel and frames per segment; a.scale; a.window (N floats or nullptr).
+// CARRY (streaming synthesis, fft_stft_stream_synthesize): one item per channel (a.nseg = 1, a.seg_frames = a.inner) and no halo;
+// the accumulators start from, and end in, `carry` + c (N - hop) / 2: the N - hop samples after the call's last hop, as float2
+// [i][j] (sample pair i T + j of the carried span, so the load and the store are coalesced).  The sums are formed in the same
+// order as in one unsegmented run, so the signal does not depend on how the frames are split into calls.
 // ---------------------------------------------------------------------------------------------
-template <int LOGM, int HQ, int LOGW>
-FFT_HD void ristft_body (const FftArgs& a)
+template <int LOGM, int HQ, int LOGW, bool CARRY = false>
+FFT_HD void ristft_body (const FftArgs& a, float2* __restrict__ carry = nullptr)
 {
     constexpr int R = 16;
     using G = Geo<LOGM, R>;
@@ -1702,10 +1706,11 @@ FFT_HD void ristft_body (const FftArgs& a)
     const float2* __restrict__ win2 = reinterpret_cast<const float2*> (a.window);
     const float2 scale2 = make_float2 (a.scale, a.scale);
     float2 acc[NACC];
+    float2* __restrict__ st = CARRY ? carry + (long long) c * (NACC * T) + j : nullptr;
 #pragma unroll
     for (int i = 0; i < NACC; ++i)
-        acc[i] = make_float2 (0.f, 0.f);
-    const int f_first = UNIFORM ? fs - HALO : (fs - HALO > 0 ? fs - HALO : 0);
+        acc[i] = CARRY ? st[i * T] : make_float2 (0.f, 0.f);
+    const int f_first = CARRY ? fs : UNIFORM ? fs - HALO : (fs - HALO > 0 ? fs - HALO : 0);
     const int f_last = UNIFORM ? fs + a.seg_frames : fe;
     for (int ff = f_first; ff < f_last; ++ff)
     {
@@ -1738,12 +1743,18 @@ FFT_HD void ristft_body (const FftArgs& a)
 #pragma unroll
         for (int i = 0; i < NACC; ++i)
             acc[i] = i + HQ < NACC ? f2_add (acc[i + HQ], v[i + HQ]) : v[i + HQ];
-        if (f + 1 == fe && fe == frames) // end of the channel: the carried samples are output too
+        if (! CARRY && f + 1 == fe && fe == frames) // end of the channel: the carried samples are output too
         {
 #pragma unroll
             for (int i = 0; i < NACC; ++i)
                 o[HOP2 + T * i] = acc[i];
         }
+    }
+    if (CARRY && item_ok)
+    {
+#pragma unroll
+        for (int i = 0; i < NACC; ++i)
+            st[i * T] = acc[i];
     }
 }
 #ifndef CFB_RISTFT_MINB
@@ -1753,6 +1764,11 @@ template <int LOGM, int HQ, int LOGW>
 __global__ void __launch_bounds__ (Launch<LOGM, 16>::THREADS, CFB_RISTFT_MINB) ristft_kernel (const FftArgs a)
 {
     ristft_body<LOGM, HQ, LOGW> (a);
+}
+template <int LOGM, int HQ, int LOGW>
+__global__ void __launch_bounds__ (Launch<LOGM, 16>::THREADS, CFB_RISTFT_MINB) ristft_carry_kernel (const FftArgs a, float2* carry)
+{
+    ristft_body<LOGM, HQ, LOGW, true> (a, carry);
 }
 
 template <int LOGM, int R, int LOGW>

@@ -135,6 +135,37 @@ int fft_convolver_reset (void* ctx, void* stream);
 int fft_convolver_segments (void* ctx, int* block_sizes, int* partitions, int max_segments);
 int fft_convolver_destroy (void* ctx);
 
+/* Streaming STFT of `channels` real signals for real-time spectral processing (denoisers, spectral gates, vocoders): a stateful
+   context that turns hop new samples per channel into one spectrum (analysis), and one spectrum into hop finished samples
+   (overlap-add synthesis), `frames` at a time, keeping its own input history and overlap-add tail.
+     fft_stft_stream_create      setup: a REAL power-of-two plan with 128 <= N <= 8192 (the context keeps its own copy; the setup
+                                 may be destroyed afterwards); hop = N/2, N/4 or N/8; 1 <= frames <= max_frames on every call.
+                                 The windows (N floats, host or device, NULL = rectangular) are copied: the caller may free them
+                                 when create returns.  Spectra in the plan's ordered (ordered != 0) or unordered layout,
+                                 synthesis scaled by `scale`.  Allocates and zeroes all state; synchronous on `stream`.
+     fft_stft_stream_analyze     consumes frames * hop samples per channel at input + c*input_stride (8-byte aligned, even
+                                 stride) and writes `frames` spectra at spectra + c*spec_channel_stride + f*spec_frame_stride
+     fft_stft_stream_synthesize  reads `frames` spectra (same layout) and writes frames * hop samples per channel at
+                                 output + c*output_stride (8-byte aligned, even stride)
+     fft_stft_stream_reset       back to silence: both frame counts to zero
+     fft_stft_stream_destroy     waits for the device, then frees the context
+   Analysis: with x_c the samples passed to analyze for channel c since create / reset, preceded by N - hop zeros, the j-th
+   spectrum is frame j of fft_stft_forward on x_c: the forward transform of analysis_window * x_c[j hop, j hop + N), bit for bit.
+   Synthesis: with S_j the j-th spectrum passed to synthesize since create / reset, the concatenated output is the first J hop
+   samples of fft_istft_overlap_add (S_0 .. S_{J-1}, hop, synthesis_window, scale) -- the samples no later frame reaches --
+   bit-identical however the frames are split into calls.  Analysis followed by synthesis returns the input delayed by N - hop,
+   scaled by the window-overlap sum.  The two directions keep independent frame counts; a context may be used for one only.
+   Spectrum alignment as for fft_istft_overlap_add (8-byte, 16-byte for unordered spectra).  Device pointers only; analyze,
+   synthesize and reset are stream-ordered, allocate nothing and do not block the host.  Calls on one context must be ordered
+   on one stream, on the device that was current at create, and a context must not be used from two threads at the same time.
+   A bad argument returns FFT_B200_EINVAL and leaves the context unchanged. */
+int fft_stft_stream_create (void* setup, int channels, long long hop, int max_frames, const float* analysis_window, const float* synthesis_window, float scale,
+                            int ordered, void* stream, void** ctx_out);
+int fft_stft_stream_analyze (void* ctx, const float* input, long long input_stride, int frames, float* spectra, long long spec_channel_stride, long long spec_frame_stride, void* stream);
+int fft_stft_stream_synthesize (void* ctx, const float* spectra, long long spec_channel_stride, long long spec_frame_stride, int frames, float* output, long long output_stride, void* stream);
+int fft_stft_stream_reset (void* ctx, void* stream);
+int fft_stft_stream_destroy (void* ctx);
+
 /* Distributed four-step transform of ONE complex transform of N = 2^n >= 2^21 points over `world` GPUs
    (one process per GPU): the three LOCAL phases; the exchange between phase 0 and phase 1 is an
    all-to-all of equal contiguous chunks (NCCL, or peer stores, see fft_dist_phase0_peer).
