@@ -533,6 +533,23 @@ FFT_HD int unordered_pos_real (int bin, int logW)
     return ((((b << logW) + r) * 2) << logW) + lane;
 }
 
+// Twiddles W^(j q), q = 1 .. r-1, of a short last stage with 32 points per thread: rows q = 1, 2, 3 and 4, 8, .. come
+// from load (q), every other power is one product w^(q mod 4) w^(q - q mod 4), as in the full-radix stages.
+// pipe_kernel keeps only the loaded rows in shared memory; fft_kernel forms the same products, so a transform gives
+// the same bits in either kernel.
+template <int r, class Load>
+FFT_HD void last_stage_tw (float2 (&w)[r], const Load& load)
+{
+#pragma unroll
+    for (int q = 1; q < r; ++q)
+        if (q < 4 || (q & 3) == 0)
+            w[q] = load (q);
+#pragma unroll
+    for (int q = 5; q < r; ++q)
+        if ((q & 3) != 0)
+            w[q] = cmul_dir<-1> (w[q & 3], w[q & ~3]);
+}
+
 // ---------------------------------------------------------------------------------------------
 // one Stockham stage on the thread's R registers.  On entry v[m] = x_s[j + m T] (x_s = stage input in
 // natural order); on exit of the last stage v[m] = X[j + m T].
@@ -578,6 +595,24 @@ FFT_HD void stage_compute (float2 (&v)[G::R], int j, const float2* __restrict__ 
             v[4 * a4 + 1] = cmul_dir<DIR> (v[4 * a4 + 1], cmul_dir<-1> (w1, wa));
             v[4 * a4 + 2] = cmul_dir<DIR> (v[4 * a4 + 2], cmul_dir<-1> (w2, wa));
             v[4 * a4 + 3] = cmul_dir<DIR> (v[4 * a4 + 3], cmul_dir<-1> (w3, wa));
+        }
+    }
+    else if constexpr (STAGE > 0 && G::R == 32)
+    {
+        // last stage, radix r < R, 32 points per thread: the twiddles of pipe_kernel (last_stage_tw), so that the two
+        // kernels give the same bits at the sizes both serve
+        const float2* __restrict__ t = tw + G::tw_off (STAGE) + j;
+        float2 w[r];
+        last_stage_tw<r> (w, [&] (int q) { return __ldg (t + (q - 1) * G::T); });
+#pragma unroll
+        for (int q = 1; q < r; ++q)
+        {
+#pragma unroll
+            for (int u = 0; u < SUB; ++u)
+            {
+                const float2 x = cmul_dir<DIR> (v[u + q * SUB], w[q]);
+                v[u + q * SUB] = mul_w32_rt<DIR> (x, u * q);
+            }
         }
     }
     else if constexpr (STAGE > 0)
@@ -936,7 +971,10 @@ FFT_HD void fft_core (const float* __restrict__ in, float* __restrict__ out, boo
     // points, and loses 1.5 % for unordered 2^12 and 6 % in the warp-pipelined kernel (landing-buffer input), which keep the table.
     // Not below 2^11 complex points (gains of 0..3 % there): those sizes also run in the warp-pipelined kernels, and the host- and
     // device-pointer paths of the STFT entry points, which may pick different kernels, promise bit-identical results.
-    constexpr bool RTW_DERIVE = CFB_REAL_TW_DERIVE == 1 || (CFB_REAL_TW_DERIVE == 2 && IN_UNION == 0 && LOGM >= 11 && (! UNORD || LOGM <= 11));
+    // The sizes pipe_kernel also serves (32 points per thread at 2^13 / 2^14) derive them in every layout, as pipe_kernel does: a
+    // batch gives the same bits whichever of the two kernels its geometry selects.
+    constexpr bool RTW_DERIVE = CFB_REAL_TW_DERIVE == 1
+                                || (CFB_REAL_TW_DERIVE == 2 && IN_UNION == 0 && LOGM >= 11 && (! UNORD || LOGM <= 11 || (R == 32 && LOGM >= 13)));
     float* sf = reinterpret_cast<float*> (s); // the same buffer seen as the unordered staging image
     constexpr int logW = LOGW;
     struct { const float2* tw; const float2* rtw; } a { tw_, rtw_ };

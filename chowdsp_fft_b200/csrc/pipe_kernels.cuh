@@ -70,6 +70,7 @@ struct PipeGeo
     static_assert (SMEM_BYTES <= 227 * 1024, "landing + exchange buffers exceed the shared memory of an SM");
     static_assert (RL >= 4, "expects a short last stage of radix >= 4");
     static FFT_CX int tw_row_q (int i) { return i < 3 ? i + 1 : 4 * (i - 2); } // smem row i holds power q
+    static FFT_CX int tw_row_of (int q) { return q < 4 ? q - 1 : q / 4 + 2; }  // its inverse (q < 4 or q % 4 == 0)
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -623,13 +624,7 @@ FFT_HD void pipe_last_stage (float2 (&v)[32], int j, const float2* tws)
     constexpr int r = P::RL, SUB = 32 / r, T = G::T;
     float2 w[r];
     const float2* tj = tws + j;
-#pragma unroll
-    for (int i = 0; i < P::TW_ROWS; ++i)
-        w[P::tw_row_q (i)] = lds2 (tj + i * T);
-#pragma unroll
-    for (int q = 5; q < r; ++q)
-        if ((q & 3) != 0)
-            w[q] = cmul_dir<-1> (w[q & 3], w[q & ~3]);
+    last_stage_tw<r> (w, [&] (int q) { return lds2 (tj + P::tw_row_of (q) * T); });
 #pragma unroll
     for (int q = 1; q < r; ++q)
     {
@@ -734,42 +729,11 @@ FFT_HD void pipe_body (const FftArgs& a)
             for (int m = 0; m < R; ++m)
                 v[m] = staged_load (lf, up.cplx (m), WL);
         }
-        else if constexpr (! P::IN_UNORD)
-        {
-            // merge step  Z'[k] = (X[k] + X*[M-k]) + i conj(w_k) (X[k] - X*[M-k]),  w_k = e^{-2 pi i k / 2M}: both
-            // operands come straight from the landing buffer, so each thread forms all of its own k = j + m T.
-            // For k >= M/2, w_k = -i w_{k - M/2}: the table only holds k < M/2 (times 1/2).
-            const float2* lj = land + j;
-            const float2 two = make_float2 (2.f, 2.f);
-#pragma unroll
-            for (int m = 0; m < R / 2; ++m)
-            {
-                const float2 wh = real_tw<32, kPipeDeriveRtw> (wj, a.rtw + j + m * T, m);
-                {
-                    const float2 xa = lds2 (lj + m * T);
-                    const float2 xm = lds2 ((m == 0 && j == 0) ? land : land + (M - m * T) - j);
-                    const float2 cm = make_float2 (xm.x, -xm.y);
-                    const float2 e = f2_add (xa, cm), d = f2_sub (xa, cm);
-                    const float2 wd = cmul_dir<+1> (d, wh);                       // conj(w_k) d / 2
-                    float2 zk = f2_fma (make_float2 (-wd.y, wd.x), two, e);      // e + i conj(w_k) d
-                    if (m == 0 && j == 0)
-                        zk = make_float2 (xa.x + xa.y, xa.x - xa.y);             // Z'[0] from (DC, Nyquist)
-                    v[m] = zk;
-                }
-                {
-                    const float2 xa = lds2 (lj + (m + R / 2) * T);
-                    const float2 xm = lds2 (land + (M / 2 - m * T) - j);          // M - k, k = j + m T + M/2
-                    const float2 cm = make_float2 (xm.x, -xm.y);
-                    const float2 e = f2_add (xa, cm), d = f2_sub (xa, cm);
-                    const float2 wd = cmul_dir<+1> (d, wh);                       // conj(w_{k - M/2}) d / 2
-                    v[m + R / 2] = f2_fma (wd, make_float2 (-2.f, -2.f), e);     // i * (i conj(w') d) = - conj(w') d
-                }
-            }
-        }
         else
         {
-            // unordered half spectrum: the pair (k, M-k), k = j + m T < M/2, comes from the staging image; Z'[k] is
-            // this thread's register m, Z'[M-k] belongs to thread T-j and crosses the exchange region
+            // merge step  Z'[k] = (X[k] + X*[M-k]) + i conj(w_k) (X[k] - X*[M-k]),  w_k = e^{-2 pi i k / 2M}, as fft_kernel
+            // forms it (same bits): the pair (k, M-k), k = j + m T < M/2, comes from the landing buffer (ordered) or the
+            // staging image; Z'[k] is this thread's register m, Z'[M-k] belongs to thread T-j and crosses the exchange region
             const float* lf = reinterpret_cast<const float*> (land);
             const float2 two = make_float2 (2.f, 2.f);
             __syncthreads(); // the previous iteration's last round_gather is done everywhere: xh may be overwritten
@@ -777,8 +741,17 @@ FFT_HD void pipe_body (const FftArgs& a)
             for (int m = 0; m < R / 2; ++m)
             {
                 const bool special = (m == 0 && j == 0);
-                const float2 xa = staged_load (lf, up.real_lo (m), WL);
-                const float2 xm = staged_load (lf, special ? W_HALF_ROW<3>() : up.real_hi (m), WL);
+                float2 xa, xm;
+                if constexpr (P::IN_UNORD)
+                {
+                    xa = staged_load (lf, up.real_lo (m), WL);
+                    xm = staged_load (lf, special ? W_HALF_ROW<3>() : up.real_hi (m), WL);
+                }
+                else
+                {
+                    xa = lds2 (land + j + m * T);
+                    xm = lds2 (special ? land + M / 2 : land + (M - m * T) - j);
+                }
                 const float2 wh = real_tw<32, kPipeDeriveRtw> (wj, a.rtw + j + m * T, m);
                 const float2 cm = make_float2 (xm.x, -xm.y);
                 const float2 e = f2_add (xa, cm), d = f2_sub (xa, cm);

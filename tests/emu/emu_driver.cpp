@@ -479,8 +479,8 @@ int emu_wpipe (int logM, int radix, int kind, int unord, int logW, const float* 
     int rc = -1;
     const int lw = unord ? logW : 0;
 #define CFB_EMU_WP(M, RR, K, W) if (logM == M && radix == RR && kind == K && lw == W) rc = run (integral_constant<int, M> {}, integral_constant<int, RR> {}, integral_constant<int, K> {}, integral_constant<int, W> {});
-    CFB_EMU_WP (10, 32, R2C, 0) CFB_EMU_WP (10, 32, R2C, 3) CFB_EMU_WP (10, 32, R2C, 2) CFB_EMU_WP (10, 32, C2C_FWD, 0) CFB_EMU_WP (10, 32, C2C_FWD, 3)
-    CFB_EMU_WP (9, 16, R2C, 0) CFB_EMU_WP (9, 16, R2C, 3) CFB_EMU_WP (9, 16, C2C_FWD, 0) CFB_EMU_WP (9, 16, C2C_FWD, 2)
+    CFB_EMU_WP (10, 32, R2C, 0) CFB_EMU_WP (10, 32, R2C, 3) CFB_EMU_WP (10, 32, R2C, 2) CFB_EMU_WP (10, 32, C2C_FWD, 0) CFB_EMU_WP (10, 32, C2C_FWD, 3) CFB_EMU_WP (10, 32, C2C_FWD, 2)
+    CFB_EMU_WP (9, 16, R2C, 0) CFB_EMU_WP (9, 16, R2C, 3) CFB_EMU_WP (9, 16, R2C, 2) CFB_EMU_WP (9, 16, C2C_FWD, 0) CFB_EMU_WP (9, 16, C2C_FWD, 3) CFB_EMU_WP (9, 16, C2C_FWD, 2)
 #undef CFB_EMU_WP
     if (stats)
     {

@@ -134,6 +134,57 @@ def test_emulated_pipelined_kernel(emu, oracle_mod, N, is_c, ordered):
     assert st[1] <= 1.05 * st[2] and st[3] <= 200, list(st)
 
 
+def same_bits(a, b):
+    return np.array_equal(np.ascontiguousarray(a, np.float32).view(np.uint32), np.ascontiguousarray(b, np.float32).view(np.uint32))
+
+
+@pytest.mark.parametrize("N,is_c", [(8192, True), (16384, True), (16384, False), (32768, False)])
+def test_pipelined_kernel_bit_equal_to_fft_kernel(emu, N, is_c):
+    """pipe_kernel and fft_kernel<LOGM, 32> serve the same sizes, and the dispatcher picks between them by batch geometry
+    (two-level batches, row strides, alignment): a batch must give the bits of a loop of single calls whichever kernel
+    runs, so the two must agree bit for bit.  Every kind, ordered and 8-lane unordered, 3 rows on 2 CTAs (one CTA loops)."""
+    nfl = 2 * N if is_c else N
+    logM = int(np.log2(N)) - (0 if is_c else 1)
+    batch = 3
+    rng = np.random.default_rng(N + 13)
+    x = rng.uniform(-1, 1, (batch, nfl)).astype(np.float32)
+    emu.emu_set_radix(32)
+    try:
+        for ordered in (True, False):
+            for backward in (False, True):
+                kind = (1 if backward else 0) if is_c else (3 if backward else 2)
+                p = np.zeros_like(x)
+                assert emu.emu_pipe(logM, kind, int(not ordered), x.ctypes.data_as(fp), p.ctypes.data_as(fp), batch, 2, 0, None) == 0
+                f, _ = run_fft(emu, x, N, is_c, 8, backward, ordered, batch)
+                diff = int((p.reshape(-1) != f).sum())
+                assert same_bits(p.reshape(-1), f), f"ordered={ordered} backward={backward}: {diff} of {f.size} floats differ"
+    finally:
+        emu.emu_set_radix(16)
+
+
+@pytest.mark.parametrize("N,is_c", [(512, True), (1024, True), (1024, False), (2048, False)])
+def test_warp_pipelined_kernel_bit_equal_to_fft_kernel(emu, N, is_c):
+    """wpipe_kernel takes plain batches of its sizes (unordered R2C 2048 from 4096 rows on) where fft_kernel takes smaller
+    ones: at the same points per thread the two must agree bit for bit.  Forward kinds, every layout."""
+    nfl = 2 * N if is_c else N
+    logM = int(np.log2(N)) - (0 if is_c else 1)
+    radix = 32 if logM == 10 else 16
+    batch = 5
+    rng = np.random.default_rng(N + 17)
+    x = rng.uniform(-1, 1, (batch, nfl)).astype(np.float32)
+    emu.emu_set_radix(radix)
+    try:
+        for ordered, W in ((True, 8), (False, 8), (False, 4)):
+            w = np.zeros_like(x)
+            rc = emu.emu_wpipe(logM, radix, 0 if is_c else 2, int(not ordered), {8: 3, 4: 2}[W], x.ctypes.data_as(fp), w.ctypes.data_as(fp),
+                               1, batch, 0, nfl, 0, nfl, None, 2, 2, 0, None)
+            assert rc == 0
+            f, _ = run_fft(emu, x, N, is_c, W, False, ordered, batch)
+            assert same_bits(w.reshape(-1), f), f"ordered={ordered} W={W}: {int((w.reshape(-1) != f).sum())} floats differ"
+    finally:
+        emu.emu_set_radix(16)
+
+
 def test_emulated_impulse_and_tone_positions(emu, oracle_mod):
     """Unit impulses and single-bin tones expose index / sign / layout errors exactly."""
     o = oracle_mod
