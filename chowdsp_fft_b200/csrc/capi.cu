@@ -684,11 +684,14 @@ struct LaneSet
     }
 };
 
-// keep freed scratch cached in the stream-ordered pool instead of returning it to the OS at every synchronisation
+// keep freed scratch cached in the stream-ordered pool instead of returning it to the OS at every synchronisation.  The
+// release threshold belongs to the device's default pool, so it is set once per device for the whole process, at setup
+// time (preload_large): setting it inside a stream capture invalidates the capture, so a multi-pass call must find it set
+// even on a thread that never made one before
+std::atomic<bool> g_pool_kept[kMaxDevices] {};
 void keep_pool_memory (int dev)
 {
-    static thread_local int pool_ready_for = -1;
-    if (pool_ready_for == dev)
+    if (dev < 0 || dev >= kMaxDevices || g_pool_kept[dev].load (std::memory_order_acquire))
         return;
     cudaMemPool_t pool = nullptr;
     if (cudaDeviceGetDefaultMemPool (&pool, dev) == cudaSuccess)
@@ -697,7 +700,7 @@ void keep_pool_memory (int dev)
         (void) cudaMemPoolSetAttribute (pool, cudaMemPoolAttrReleaseThreshold, &keep);
     }
     (void) cudaGetLastError();
-    pool_ready_for = dev;
+    g_pool_kept[dev].store (true, std::memory_order_release);
 }
 
 int tile_radix_for (int logL) { return (tile_radix32() != 0 && logL >= 9) ? 32 : 16; } // must match launch_tile_l (large_inst.cu)
@@ -720,6 +723,7 @@ int preload_large (Plan* p)
 {
     int dev = 0;
     CFB_CUDA (cudaGetDevice (&dev));
+    keep_pool_memory (dev);
     LargeTables lt;
     int rc = large_tables (p, dev, choose_factors (p->logM), lt);
     if (rc == 0 && p->is_complex && has_cluster (p->logM))

@@ -12,6 +12,19 @@
  * `stream` and returns.  When the data pointers are host memory the call stages chunks through the
  * device on internal streams (H2D, transform, D2H overlapped) and returns after the result is in the
  * host buffer.  Mixing host and device data pointers in one call is rejected.
+ *
+ * Streams: `stream` may be NULL, cudaStreamLegacy, cudaStreamPerThread or any created stream, blocking or not; every
+ * launch, copy and memset of a call goes to it, and helper streams of the multi-pass schedules are joined back into it
+ * before the call returns.  A plan may be used from several threads at once, each on its own stream.
+ * CUDA graphs: the stateless device-pointer calls (fft_transform_batched / _strided, fft_stft_forward,
+ * fft_istft_overlap_add, fft_juce_*_batched, fft_convolve_unordered_batched, fft_accumulate_batched,
+ * fft_partitioned_convolve_step) may be captured (global capture mode) and replayed, with no eager warm-up, from any
+ * thread: setup uploads the tables and sets the device memory pool's release threshold, so a call makes no
+ * capture-illegal API call.  Exception: the first call of a plan on a device other than the one it was created on
+ * builds that device's tables with blocking allocations; make it eagerly.  The streaming contexts (fft_convolver_*,
+ * fft_stft_stream_*) keep their block / frame counts on the host, so a replayed capture would repeat one block: they
+ * are not replayable.
+ * tests/test_gpu_streams.py checks all of this against float64 and against calls on the default stream.
  */
 #pragma once
 #include "chowdsp_fft.h"
